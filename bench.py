@@ -21,6 +21,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -28,6 +29,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the checkout, not even __pycache__ of the package it imports
+sys.dont_write_bytecode = True
 
 # algorithmic bytes per grid point per tile-frame of THIS design (DESIGN.md §5): K1 reads the 16-byte h0 record
 # and writes the Hermitian-packed intermediate W (4 packed fields x 4 B); K2h re-reads packed field 0 (4 B) for the
@@ -181,6 +184,63 @@ def step_times(wl, step):
     return (np.arange(i0, i0 + f, dtype=np.float32) * np.float32(wl["dt"])), None
 
 
+# ----------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed in its last step, so that two builds can be compared output for output.
+# The inputs are seeded (gauss(), tile_params(), step_times()), so the same arguments give the same inputs every run.
+DUMP_TEXELS = 1 << 20      # sampled texels per map: 2 maps x 16 MB + 3 x 4 MB of coordinates
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_sample(frames, rows, cols, seed=0):
+    """Fixed, seeded sample of texel coordinates (frame, row, col), sorted, of `frames` maps of rows x cols."""
+    total = frames * rows * cols
+    rng = np.random.default_rng(seed)
+    idx = np.unique(rng.integers(0, total, size=min(DUMP_TEXELS, total), dtype=np.int64))
+    return np.unravel_index(idx, (frames, rows, cols))
+
+
+def write_dump(out_dir, arrays):
+    arrays = {k: np.ascontiguousarray(v) for k, v in arrays.items()}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_batch(ws, frames, out_dir):
+    """Device slots 0..frames-1 after compute_batch: the height statistics of every tile-frame (amplitude, min, max),
+    and both RGBA32F maps at a seeded sample of texels (sample_frame = slot, sample_row, sample_col)."""
+    from watersurfacerendering_b200 import _lib as L
+    n = ws.GetTileSize()
+    a, mn, mx = ws.read_heights(0, frames)
+    f, r, c = dump_sample(frames, n, n)
+    bounds = np.searchsorted(f, np.arange(frames + 1))
+    out = {"amplitude": a, "min_height": mn, "max_height": mx, "sample_frame": f.astype(np.float32),
+           "sample_row": r.astype(np.float32), "sample_col": c.astype(np.float32)}
+    for name, which in (("displacement", L.WSO_MAP_DISPLACEMENT), ("normal", L.WSO_MAP_NORMAL)):
+        texels = np.empty((f.size, 4), np.float32)
+        for s in range(frames):
+            lo, hi = bounds[s], bounds[s + 1]
+            if hi > lo:
+                texels[lo:hi] = ws.copy_map(which, s)[r[lo:hi], c[lo:hi]]
+        out[name] = texels
+    write_dump(out_dir, out)
+
+
+def dump_slab(b, out_dir):
+    """The same for the slab path: this rank's rows of the one N x N tile-frame (sample_row = global row)."""
+    from watersurfacerendering_b200 import _lib as L
+    amp, mn, mx = b.read_heights()
+    _, r, c = dump_sample(1, 2 * b.hl, b.n)
+    out = {"amplitude": np.array([amp], np.float32), "min_height": np.array([mn], np.float32),
+           "max_height": np.array([mx], np.float32), "sample_frame": np.zeros(r.size, np.float32),
+           "sample_row": b.row_index()[r].astype(np.float32), "sample_col": c.astype(np.float32)}
+    for name, which in (("displacement", L.WSO_MAP_DISPLACEMENT), ("normal", L.WSO_MAP_NORMAL)):
+        out[name] = b.local_rows(which)[r, c]
+    write_dump(out_dir, out)
+
+
 def run_reference_arm(args, wl, rank, world):
     if rank != 0:
         return
@@ -312,6 +372,8 @@ def run_slab(args, wl, rank, world, local_rank):
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     amp, mn, mx = b.read_heights()
+    if args.dump_outputs and rank == 0:
+        dump_slab(b, args.dump_outputs)
 
     # ---- per-phase device time (events around every phase; same steps again)
     names = ["K1", "exchange", "K2h", "allreduce", "K2"]
@@ -478,8 +540,10 @@ def local_step_times(wl, step, mine):
     return step_times(wl, step)
 
 
-def bench_workload(name, wl, steps, warmup, rank, world, local_rank, *, want_e2e=True, e2e_frames=0, clocks=True):
-    """One workload on this rank's GPU: device-resident throughput, per-kernel times, end-to-end through host buffers."""
+def bench_workload(name, wl, steps, warmup, rank, world, local_rank, *, want_e2e=True, e2e_frames=0, clocks=True,
+                   dump_dir=None):
+    """One workload on this rank's GPU: device-resident throughput, per-kernel times, end-to-end through host buffers.
+    dump_dir: rank 0 writes the outputs of the last timed step there (dump_batch)."""
     import torch
     import torch.distributed as dist
     import watersurfacerendering_b200 as W
@@ -537,6 +601,8 @@ def bench_workload(name, wl, steps, warmup, rank, world, local_rank, *, want_e2e
     clk = sampler.stop() if (rank == 0 and sampler) else None
     frames_all = reduce_ranks(float(F), dist.ReduceOp.SUM)   # tile-frames per step over all ranks
     value = frames_all * steps / (ms * 1e-3)
+    if dump_dir and rank == 0:
+        dump_batch(ws, F, dump_dir)
 
     # ---- per-kernel timing (same steps again, CUDA events around every launch) -----------------------
     ws.set_profiling(True)
@@ -696,12 +762,14 @@ def c1_latency(local_rank):
            "back_to_back_us_python_binding": e0.elapsed_time(e1) * 1e3 / frames,
            "host_enqueue_us_python_binding": (c1 - c0) * 1e6 / frames}
     ws.close()
-    exe = os.path.join(ROOT, "tools", "lat_bench")
     try:
-        if not os.path.exists(exe):
-            subprocess.run(["make", "-C", os.path.join(ROOT, "examples"), "lat_bench"], capture_output=True, timeout=120)
-        r = subprocess.run([exe, str(n), "2000"], capture_output=True, text=True, timeout=120,
-                           env=dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", str(local_rank))))
+        # built outside the tree: the benchmark leaves the checkout untouched (it may be read-only)
+        with tempfile.TemporaryDirectory(prefix="wso_lat_bench_") as tmp:
+            exe = os.path.join(tmp, "lat_bench")
+            subprocess.run(["make", "-C", os.path.join(ROOT, "examples"), "lat_bench", f"LAT_BENCH={exe}"],
+                           capture_output=True, timeout=120)
+            r = subprocess.run([exe, str(n), "2000"], capture_output=True, text=True, timeout=120,
+                               env=dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", str(local_rank))))
         out["c_abi"] = json.loads(r.stdout.strip().splitlines()[-1])
     except Exception as ex:
         out["c_abi"] = {"unavailable": repr(ex)[:200]}
@@ -721,7 +789,14 @@ def main():
     ap.add_argument("--slab-fused", type=int, default=1,
                     help="c5: 1 = exchange kernel with direct peer stores over NVLink, 3 = the same issued field by field on "
                          "a second stream behind K1, 0 = exchange kernel into send blocks + NCCL all-to-all")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0: height statistics of every "
+                         "tile-frame, a seeded sample of the displacement and normal maps) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     wl = dict(WORKLOADS[args.workload])
@@ -749,7 +824,8 @@ def main():
         return
 
     n = wl["n"]
-    res = bench_workload(args.workload, wl, args.steps, args.warmup, rank, world, local_rank, e2e_frames=args.e2e_frames)
+    res = bench_workload(args.workload, wl, args.steps, args.warmup, rank, world, local_rank, e2e_frames=args.e2e_frames,
+                         dump_dir=args.dump_outputs)
 
     # ---- the north-star targets that the headline workload does not show, measured in the same run -----------
     targets = None

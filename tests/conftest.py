@@ -14,8 +14,21 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
+class GoldenCase(dict):
+    """The arrays of one fixture case; ``files`` lists their names like np.load's NpzFile."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
 def load_golden(name):
-    g = np.load(os.path.join(GOLDEN, name + ".npz"))
+    """One case, merged from <name>.npz and its parts <name>.1.npz, ... (make_golden.py keeps each file under 1 MB)."""
+    g = GoldenCase()
+    for f in sorted(os.listdir(GOLDEN)):
+        if f == name + ".npz" or (f.startswith(name + ".") and f.endswith(".npz")):
+            with np.load(os.path.join(GOLDEN, f)) as z:
+                g.update((k, z[k]) for k in z.files)
     p = g["params"]
     params = dict(tile_size=int(p[0]), tile_length=float(p[1]), wind_x=float(p[2]), wind_y=float(p[3]),
                   wind_speed=float(p[4]), phillips_const=float(p[5]), damping=float(p[6]),

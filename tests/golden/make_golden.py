@@ -7,9 +7,11 @@ its own for this path (SURVEY.md §4), so these files are the pinned outputs of 
 
     python tests/golden/make_golden.py
 
-Each case -> one .npz:  params, seed, xi (Gaussian array), h0 (N,N,5 fp32: the reference's 20-byte
-record), wave_vectors, t[], A[], minh[], maxh[], disp[t], norm[t], and (small N) the pre-FFT spectra.
+Each case -> params, seed, xi (Gaussian array), h0 (N,N,5 fp32: the reference's 20-byte record), wave_vectors,
+t[], A[], minh[], maxh[], disp[t], norm[t], and (small N) the pre-FFT spectra, packed into <name>.npz, <name>.1.npz, ...
+so that every file stays under 1 MB (tests/conftest.py load_golden() merges them).
 """
+import io
 import os
 import sys
 
@@ -20,6 +22,35 @@ sys.path.insert(0, ROOT)
 from oracle import refmodel as R  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
+PART_BYTES = 990_000   # bytes per file (each array measured as its own .npz, headers included): below 1 MB
+
+
+def _compressed_size(key, a):
+    buf = io.BytesIO()
+    np.savez_compressed(buf, **{key: a})
+    return buf.tell()
+
+
+def save_case(name, arrays):
+    """Pack the arrays of one case, in order, into as few files of at most PART_BYTES as fit."""
+    parts, size = [{}], 0
+    for key, a in arrays.items():
+        n = _compressed_size(key, a)
+        if n > PART_BYTES:
+            raise ValueError(f"{name}/{key}: {n} bytes compressed does not fit one file")
+        if parts[-1] and size + n > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][key] = a
+        size += n
+    for f in os.listdir(OUT):
+        if f.startswith(name + ".") and f.endswith(".npz"):
+            os.remove(os.path.join(OUT, f))
+    for i, part in enumerate(parts):
+        path = os.path.join(OUT, name + (f".{i}" if i else "") + ".npz")
+        np.savez_compressed(path, **part)
+        print(path, os.path.getsize(path) // 1024, "KiB")
+
 
 CASES = [
     # name, N, L, wind, V, A, damping, T, lambda, seed, times, with_spectra
@@ -68,9 +99,7 @@ def main():
                    maxh=np.array(maxs, np.float32), disp=np.stack(disps), norm=np.stack(norms))
         if with_spec:
             out["spectra"] = np.stack(specs)
-        path = os.path.join(OUT, name + ".npz")
-        np.savez_compressed(path, **out)
-        print(name, os.path.getsize(path) // 1024, "KiB")
+        save_case(name, out)
 
 
 if __name__ == "__main__":
