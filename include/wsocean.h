@@ -157,6 +157,38 @@ WSO_API int wso_map_device(wso_ctx* ctx, int which, uint32_t slot, void** dptr, 
 WSO_API int wso_copy_map(wso_ctx* ctx, int which, uint32_t slot, float* dst_host);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Map format (an extension; the reference writes RGBA32F only).  Both maps of a context are in one format:
+ *   WSO_MAP_RGBA32F (default): 4 x fp32 per texel, 16 bytes, VK_FORMAT_R32G32B32A32_SFLOAT - everything above.
+ *   WSO_MAP_RGBA16F: (x, y, z, w) as 4 x IEEE binary16, little-endian, tightly packed: 8 bytes per texel,
+ *       VK_FORMAT_R16G16B16A16_SFLOAT (a mandatory sampled format with linear filtering).  Each channel is the value the
+ *       RGBA32F path computes, rounded to nearest even; magnitudes >= 65520 become +-inf, NaN stays NaN (IEEE conversion).
+ *       Half the device memory, half the device->host bytes and half of K2's stores.  disp.y is normalised to [-1, 1];
+ *       at the 512^2 defaults |lambda*Dx| <= 23 (about 1 cm of binary16 spacing there) and the normals <= 1.1.
+ * wso_set_map_format reallocates both map arrays and the pinned mirrors at the new size (in the current backing: own or
+ * exportable memory; an array imported with wso_import_external_fd returns to own memory) and resets their contents
+ * to the resize() defaults in the new format (displacement 0, normal (0, 1, 0, 0)).  Prepare() state, the tile size,
+ * the Jacobian switch and wso_set_exportable are kept; the format survives Prepare(), tile-size changes and
+ * wso_set_exportable.  Any other value: WSO_ERR_INVALID_ARG, state unchanged.
+ * Layout in either format: [slot][N*N] texels, slot s at byte s*B*N*N, row pitch B*N (B = 16 or 8 bytes per texel); this
+ * is the layout of wso_map_device, wso_export_fd (which then reports the smaller array) and of the memory
+ * wso_import_external_fd needs (max_slots*B*N*N bytes).
+ * The float-typed calls wso_map_host, wso_copy_map and wso_compute_to_host serve RGBA32F only and answer
+ * WSO_ERR_INVALID_ARG in RGBA16F; their byte-typed counterparts below work in both formats:
+ *   wso_map_host_bytes       : pinned host copy of slot 0 (as wso_map_host); *bytes = B*N*N
+ *   wso_copy_map_bytes       : blocking copy of one slot into dst_host, which must hold dst_bytes >= B*N*N
+ *   wso_compute_to_host_bytes: wso_compute_to_host into buffers of bytes_each >= n*B*N*N bytes each
+ * Not on the slab path (RGBA32F only).  RGBA16F maps always come from the CTA-per-line K2 (wso_select_kernels bit 2
+ * does not apply to them). */
+enum { WSO_MAP_RGBA32F = 0, WSO_MAP_RGBA16F = 1 };
+WSO_API int wso_set_map_format(wso_ctx* ctx, int format);
+WSO_API int wso_get_map_format(const wso_ctx* ctx, int* format);
+WSO_API int wso_map_host_bytes(wso_ctx* ctx, int which, const void** ptr, size_t* bytes);
+WSO_API int wso_copy_map_bytes(wso_ctx* ctx, int which, uint32_t slot, void* dst_host, size_t dst_bytes);
+WSO_API int wso_compute_to_host_bytes(wso_ctx* ctx, uint32_t n, const uint32_t* tiles, const float* t,
+                                      void* disp_host, void* norm_host, size_t bytes_each, float* amplitude,
+                                      float* min_height, float* max_height);
+
+/* ------------------------------------------------------------------------------------------------------------
  * External-memory interop (SURVEY row f-2): the maps land in memory a Vulkan device can bind, so the renderer's
  * vkCmdCopyBufferToImage reads them where K2 wrote them.  Replaces: the two 16*N*N-byte memcpy calls into the mapped
  * staging buffer and the PCIe upload behind them (WaterSurfaceMesh.cpp:701-755, vulkan/Texture2D.cpp:175-226).
@@ -166,9 +198,10 @@ WSO_API int wso_copy_map(wso_ctx* ctx, int which, uint32_t slot, float* dst_host
  *       { handleType = VK_EXTERNAL_MEMORY_HANDLE_TYPE_OPAQUE_FD_BIT } and binds a VkBuffer of *bytes to it.
  *       The caller owns the returned fd (close() it, or let the Vulkan import consume it).
  *   wso_import_external_fd : Vulkan allocated and exported the memory (vkGetMemoryFdKHR); the library maps
- *       [offset, offset + max_slots*16*N*N) of it as the output array of map `which`.  On success the fd belongs
+ *       [offset, offset + max_slots*16*N*N) of it as the output array of map `which` (8*N*N per slot in RGBA16F).  On success the fd belongs
  *       to CUDA.  A tile-size change (Prepare after SetTileSize) drops the import and returns to own memory.
- * Layout either way: [slot][N*N] RGBA32F texels, slot s at byte offset s*16*N*N (+ offset), row pitch 16*N.
+ * Layout either way: [slot][N*N] RGBA32F texels, slot s at byte offset s*16*N*N (+ offset), row pitch 16*N
+ * (RGBA16F maps, wso_set_map_format: 8*N*N and 8*N).
  * Map contents are reset to zero by wso_set_exportable / wso_import_external_fd; Prepare() state is kept.
  * Ordering with the renderer: wso_import_semaphore_fd binds an exported VkSemaphore (binary: is_timeline = 0,
  * timeline: 1; `index` 0 or 1); wso_signal_semaphore / wso_wait_semaphore enqueue a signal / wait on the context's
@@ -198,7 +231,8 @@ WSO_API int wso_unregister_host(void* ptr);
  * persistent form (a fixed grid of CTAs walks the work items and requests the inputs of its next item ahead of the store
  * phase of the current one; bit-identical results); -1 restores the built-in choice (what measured faster per size).
  * Any other bit: WSO_ERR_INVALID_ARG.  Process-wide; meant for A/B measurements and for the parity tests, which run
- * every form. */
+ * every form.  A context with RGBA16F maps (wso_set_map_format) runs the CTA-per-line K2 whatever bit 2 says (the
+ * warp-per-line K2 writes RGBA32F only); the K1 / K2h choice and bit 6 apply as usual. */
 WSO_API int wso_select_kernels(int mask);
 
 /* Introspection used by the benchmark: number of kernels launched so far by this context, the chunk

@@ -23,6 +23,10 @@ WSO_ERR_H0_NOT_CONJUGATE = -6
 WSO_MAP_DISPLACEMENT = 0
 WSO_MAP_NORMAL = 1
 
+# map texel formats (wso_set_map_format)
+WSO_MAP_RGBA32F = 0
+WSO_MAP_RGBA16F = 1
+
 STATUS_NAMES = {
     0: "WSO_OK", -1: "WSO_ERR_INVALID_ARG", -2: "WSO_ERR_BAD_TILE_SIZE", -3: "WSO_ERR_NOT_PREPARED",
     -4: "WSO_ERR_CUDA", -5: "WSO_ERR_OUT_OF_MEMORY", -6: "WSO_ERR_H0_NOT_CONJUGATE",
@@ -74,6 +78,12 @@ SYMBOLS = {
     "wso_map_host": (_int, [_vp, _int, C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "wso_map_device": (_int, [_vp, _int, _u32, C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "wso_copy_map": (_int, [_vp, _int, _u32, _vp]),
+    # map format (RGBA32F / RGBA16F) and the byte-typed map accessors that serve both
+    "wso_set_map_format": (_int, [_vp, _int]),
+    "wso_get_map_format": (_int, [_vp, C.POINTER(_int)]),
+    "wso_map_host_bytes": (_int, [_vp, _int, C.POINTER(_vp), C.POINTER(C.c_size_t)]),
+    "wso_copy_map_bytes": (_int, [_vp, _int, _u32, _vp, C.c_size_t]),
+    "wso_compute_to_host_bytes": (_int, [_vp, _u32, _vp, _vp, _vp, _vp, C.c_size_t, _vp, _vp, _vp]),
     # external-memory interop (Vulkan side of the maps)
     "wso_set_exportable": (_int, [_vp, _int]),
     "wso_export_fd": (_int, [_vp, _int, C.POINTER(_int), C.POINTER(C.c_size_t)]),

@@ -60,6 +60,7 @@ struct wso_ctx {
     uint32_t chunk = 1;
     bool first_use = true;
     bool jacobian = false;  // disp.w = Jacobian instead of 1.0f (wso_set_compute_jacobian, SURVEY row f-4)
+    int map_format = WSO_MAP_RGBA32F;  // texel format of both maps (wso_set_map_format); sizes: map_texel_bytes()
     uint64_t launches = 0;
     std::vector<Tile> tiles;
     // device
@@ -71,7 +72,7 @@ struct wso_ctx {
     wso::FrameGraph frame_graph;  // launch sequence of one tile-frame as an instantiated CUDA graph (wso_launch.h)
     int frame_graph_mode = 1;     // 0: plain launches, 1: graph for sizes up to 512^2, 2: graph for every size (WSO_FRAME_GRAPH)
     bool l2_policy_done = false; // WSO_EXP_L2_PERSIST_MB examined (experiment hook in wso_compute_batch)
-    float4* d_disp = nullptr;    // [slot][N*N]
+    float4* d_disp = nullptr;    // [slot][N*N] texels of map_texel_bytes() each (RGBA16F: Half4, see map_slot)
     float4* d_norm = nullptr;
     float* d_minmax = nullptr;   // [slot][2]
     float* d_ampl = nullptr;     // [slot]
@@ -81,8 +82,8 @@ struct wso_ctx {
     bool exportable = false;
     cudaExternalSemaphore_t ext_sem[2] = {nullptr, nullptr};
     // pinned host
-    float4* h_disp = nullptr;    // slot 0 mirror for wso_compute / wso_map_host
-    float4* h_norm = nullptr;
+    void* h_disp = nullptr;      // slot 0 mirror for wso_compute / wso_map_host_bytes (N*N texels in the map format)
+    void* h_norm = nullptr;
     float* h_small = nullptr;    // [small_cap][3] amplitude,min,max staging
     size_t small_cap = 0;
     std::vector<TileDev> h_tiles;
@@ -177,6 +178,14 @@ const VmmApi& vmm_api() {
 
 float4*& map_ptr(wso_ctx* c, int which) { return which == 0 ? c->d_disp : c->d_norm; }
 
+// Bytes of one map texel in the context's format: the one source for every size, offset and pitch of the map arrays,
+// their pinned mirrors and the host copies.  Slot s of a map starts at byte s * map_texel_bytes * N*N.
+size_t map_texel_bytes(const wso_ctx* c) { return c->map_format == WSO_MAP_RGBA16F ? sizeof(wso::Half4) : sizeof(float4); }
+size_t map_slot_bytes(const wso_ctx* c) { return map_texel_bytes(c) * (size_t)c->n * c->n; }
+char* map_slot(wso_ctx* c, int which, uint32_t slot) {
+    return reinterpret_cast<char*>(map_ptr(c, which)) + map_slot_bytes(c) * slot;
+}
+
 void free_map(wso_ctx* c, int which) {
     MapBacking& b = c->map_mem[which];
     float4*& p = map_ptr(c, which);
@@ -261,16 +270,27 @@ void free_device_buffers(wso_ctx* c) {
 
 // Map contents before the first ComputeWaves(): the reference's resize() defaults (WSTessendorf.cpp:48-54) -
 // displacement (0,0,0,0), normal (0,1,0,0) - in every device slot and in the pinned host mirrors of slot 0.
+// RGBA16F: the same values in binary16, normal (0, 1, 0, 0) = halves (0x0000, 0x3c00, 0x0000, 0x0000).
 int reset_map_contents(wso_ctx* c, size_t n2, int which_mask = 3) {
+    const size_t tb = map_texel_bytes(c);
     if (which_mask & 1) {
-        WSO_CUDA(c, cudaMemsetAsync(c->d_disp, 0, sizeof(float4) * n2 * c->max_slots, c->stream));
-        if (c->h_disp) std::memset(c->h_disp, 0, sizeof(float4) * n2);
+        WSO_CUDA(c, cudaMemsetAsync(c->d_disp, 0, tb * n2 * c->max_slots, c->stream));
+        if (c->h_disp) std::memset(c->h_disp, 0, tb * n2);
     }
     if ((which_mask & 2) && c->h_norm) {
-        const float4 up = make_float4(0.0f, 1.0f, 0.0f, 0.0f);
-        for (size_t i = 0; i < n2; ++i) c->h_norm[i] = up;
+        if (c->map_format == WSO_MAP_RGBA16F) {
+            const wso::Half4 up = {0x3c00u << 16, 0u};
+            wso::Half4* h = static_cast<wso::Half4*>(c->h_norm);
+            for (size_t i = 0; i < n2; ++i) h[i] = up;
+        } else {
+            const float4 up = make_float4(0.0f, 1.0f, 0.0f, 0.0f);
+            float4* h = static_cast<float4*>(c->h_norm);
+            for (size_t i = 0; i < n2; ++i) h[i] = up;
+        }
+        // (slot offsets from n2: while the buffers of a new size are allocated, c->n is still 0)
         for (uint32_t sl = 0; sl < c->max_slots; ++sl)
-            WSO_CUDA(c, cudaMemcpyAsync(c->d_norm + n2 * sl, c->h_norm, sizeof(float4) * n2, cudaMemcpyHostToDevice, c->stream));
+            WSO_CUDA(c, cudaMemcpyAsync(reinterpret_cast<char*>(c->d_norm) + tb * n2 * sl, c->h_norm, tb * n2,
+                                        cudaMemcpyHostToDevice, c->stream));
     }
     return WSO_OK;
 }
@@ -328,13 +348,13 @@ int allocate_buffers(wso_ctx* c, uint32_t n, int logn) {
     WSO_CUDA(c, cudaMalloc(&c->d_tw, sizeof(float2) * n));
     WSO_CUDA(c, cudaMalloc(&c->d_W, w_item * chunk * (size_t)(c->lanes > 2 ? c->lanes : 2)));
     for (int which = 0; which < 2; ++which) {
-        const int rc = alloc_map(c, which, sizeof(float4) * n2 * c->max_slots);
+        const int rc = alloc_map(c, which, map_texel_bytes(c) * n2 * c->max_slots);
         if (rc != WSO_OK) return rc;
     }
     WSO_CUDA(c, cudaMalloc(&c->d_minmax, sizeof(float) * 2 * c->max_slots));
     WSO_CUDA(c, cudaMalloc(&c->d_ampl, sizeof(float) * c->max_slots));
-    WSO_CUDA(c, cudaMallocHost(&c->h_disp, sizeof(float4) * n2));
-    WSO_CUDA(c, cudaMallocHost(&c->h_norm, sizeof(float4) * n2));
+    WSO_CUDA(c, cudaMallocHost(&c->h_disp, map_texel_bytes(c) * n2));
+    WSO_CUDA(c, cudaMallocHost(&c->h_norm, map_texel_bytes(c) * n2));
     c->small_cap = c->max_slots;
     WSO_CUDA(c, cudaMallocHost(&c->h_small, sizeof(float) * 3 * c->small_cap));
     {
@@ -492,8 +512,9 @@ int enqueue_chunk(wso_ctx* c, uint32_t n_items, const uint32_t* tiles, const flo
     // reach across graph launches: profiles/r3_frame_graph.md.  Mode 2 = every size.)
     const bool as_graph = n_items == 1 && ev == nullptr &&
                           (c->frame_graph_mode == 2 || (c->frame_graph_mode == 1 && c->logn <= kFrameGraphMaxLogN));
-    cudaError_t e = as_graph ? wso::launch_frame_graph(c->frame_graph, c->logn, args, stream, c->jacobian)
-                             : wso::launch_compute_waves(c->logn, args, (int)n_items, stream, c->jacobian, ev);
+    const bool half = c->map_format == WSO_MAP_RGBA16F;
+    cudaError_t e = as_graph ? wso::launch_frame_graph(c->frame_graph, c->logn, args, stream, c->jacobian, half)
+                             : wso::launch_compute_waves(c->logn, args, (int)n_items, stream, c->jacobian, half, ev);
     if (e != cudaSuccess) return fail_cuda(c, e, "kernel launch");
     c->first_use = false;
     c->launches += (uint64_t)wso::kernels_per_launch();
@@ -926,7 +947,7 @@ int wso_compute(wso_ctx* c, float t, float* amplitude) {
     WSO_CUDA(c, cudaSetDevice(c->device));
     if ((rc = push_lambdas(c)) != WSO_OK) return rc;
     if ((rc = enqueue_chunk(c, 1, nullptr, &t, 0, 0, c->stream)) != WSO_OK) return rc;
-    const size_t bytes = sizeof(float4) * (size_t)c->n * c->n;
+    const size_t bytes = map_slot_bytes(c);
     WSO_CUDA(c, cudaMemcpyAsync(c->h_disp, c->d_disp, bytes, cudaMemcpyDeviceToHost, c->stream));
     WSO_CUDA(c, cudaMemcpyAsync(c->h_norm, c->d_norm, bytes, cudaMemcpyDeviceToHost, c->stream));
     WSO_CUDA(c, cudaMemcpyAsync(c->h_small, c->d_ampl, sizeof(float), cudaMemcpyDeviceToHost, c->stream));
@@ -938,7 +959,19 @@ int wso_compute(wso_ctx* c, float t, float* amplitude) {
 int wso_compute_to_host(wso_ctx* c, uint32_t n, const uint32_t* tiles, const float* t, float* disp_host,
                         float* norm_host, float* amplitude, float* min_height, float* max_height) {
     if (!c) return WSO_ERR_INVALID_ARG;
+    if (c->map_format != WSO_MAP_RGBA32F)
+        return fail(c, WSO_ERR_INVALID_ARG, "wso_compute_to_host takes RGBA32F maps: use wso_compute_to_host_bytes");
+    return wso_compute_to_host_bytes(c, n, tiles, t, disp_host, norm_host, (size_t)n * map_slot_bytes(c), amplitude,
+                                     min_height, max_height);
+}
+
+int wso_compute_to_host_bytes(wso_ctx* c, uint32_t n, const uint32_t* tiles, const float* t, void* disp_host,
+                              void* norm_host, size_t bytes_each, float* amplitude, float* min_height,
+                              float* max_height) {
+    if (!c) return WSO_ERR_INVALID_ARG;
     if (!disp_host || !norm_host) return fail(c, WSO_ERR_INVALID_ARG, "host buffers are NULL");
+    if (bytes_each < (size_t)n * map_slot_bytes(c))
+        return fail(c, WSO_ERR_INVALID_ARG, "host buffers too small: n * N*N texels of the map format each");
     // Slots are recycled: chunk k uses slots [ (k&1)*chunk , (k&1)*chunk + m ).
     const uint32_t need = (n <= c->chunk) ? n : 2 * c->chunk;
     if (need > c->max_slots) return fail(c, WSO_ERR_INVALID_ARG, "wso_compute_to_host needs max_slots >= 2*chunk");
@@ -951,8 +984,7 @@ int wso_compute_to_host(wso_ctx* c, uint32_t n, const uint32_t* tiles, const flo
     }
     WSO_CUDA(c, cudaSetDevice(c->device));
     if ((rc = push_lambdas(c)) != WSO_OK) return rc;
-    const size_t texels = (size_t)c->n * c->n;
-    const size_t map_bytes = sizeof(float4) * texels;
+    const size_t map_bytes = map_slot_bytes(c);
     if (n > c->small_cap) {  // pinned staging for amplitude/min/max of every tile-frame
         WSO_CUDA(c, cudaStreamSynchronize(c->stream));
         cudaFreeHost(c->h_small);
@@ -978,9 +1010,9 @@ int wso_compute_to_host(wso_ctx* c, uint32_t n, const uint32_t* tiles, const flo
         if (rc != WSO_OK) return rc;
         WSO_CUDA(c, cudaEventRecord(c->ev_chunk[b], lane));
         WSO_CUDA(c, cudaStreamWaitEvent(c->copy_stream, c->ev_chunk[b], 0));
-        WSO_CUDA(c, cudaMemcpyAsync(disp_host + (size_t)done * texels * 4, c->d_disp + (size_t)slot0 * texels,
+        WSO_CUDA(c, cudaMemcpyAsync(static_cast<char*>(disp_host) + (size_t)done * map_bytes, map_slot(c, 0, slot0),
                                     map_bytes * m, cudaMemcpyDeviceToHost, c->copy_stream));
-        WSO_CUDA(c, cudaMemcpyAsync(norm_host + (size_t)done * texels * 4, c->d_norm + (size_t)slot0 * texels,
+        WSO_CUDA(c, cudaMemcpyAsync(static_cast<char*>(norm_host) + (size_t)done * map_bytes, map_slot(c, 1, slot0),
                                     map_bytes * m, cudaMemcpyDeviceToHost, c->copy_stream));
         WSO_CUDA(c, cudaMemcpyAsync(small + done, c->d_ampl + slot0, sizeof(float) * m,
                                     cudaMemcpyDeviceToHost, c->copy_stream));
@@ -1001,9 +1033,21 @@ int wso_compute_to_host(wso_ctx* c, uint32_t n, const uint32_t* tiles, const flo
 
 int wso_map_host(wso_ctx* c, int which, const float** ptr, size_t* texels) {
     if (!c || !ptr) return WSO_ERR_INVALID_ARG;
-    if (which != WSO_MAP_DISPLACEMENT && which != WSO_MAP_NORMAL) return fail(c, WSO_ERR_INVALID_ARG, "bad map id");
-    *ptr = reinterpret_cast<const float*>(which == WSO_MAP_DISPLACEMENT ? c->h_disp : c->h_norm);
+    if (c->map_format != WSO_MAP_RGBA32F)
+        return fail(c, WSO_ERR_INVALID_ARG, "wso_map_host returns RGBA32F maps: use wso_map_host_bytes");
+    const void* p = nullptr;
+    const int rc = wso_map_host_bytes(c, which, &p, nullptr);
+    if (rc != WSO_OK) return rc;
+    *ptr = static_cast<const float*>(p);
     if (texels) *texels = (size_t)c->n * c->n;
+    return WSO_OK;
+}
+
+int wso_map_host_bytes(wso_ctx* c, int which, const void** ptr, size_t* bytes) {
+    if (!c || !ptr) return WSO_ERR_INVALID_ARG;
+    if (which != WSO_MAP_DISPLACEMENT && which != WSO_MAP_NORMAL) return fail(c, WSO_ERR_INVALID_ARG, "bad map id");
+    *ptr = which == WSO_MAP_DISPLACEMENT ? c->h_disp : c->h_norm;
+    if (bytes) *bytes = map_slot_bytes(c);
     return WSO_OK;
 }
 
@@ -1011,20 +1055,26 @@ int wso_map_device(wso_ctx* c, int which, uint32_t slot, void** dptr, size_t* te
     if (!c || !dptr) return WSO_ERR_INVALID_ARG;
     if (which != WSO_MAP_DISPLACEMENT && which != WSO_MAP_NORMAL) return fail(c, WSO_ERR_INVALID_ARG, "bad map id");
     if (slot >= c->max_slots) return fail(c, WSO_ERR_INVALID_ARG, "slot out of range");
-    const size_t n2 = (size_t)c->n * c->n;
-    *dptr = (which == WSO_MAP_DISPLACEMENT ? c->d_disp : c->d_norm) + n2 * slot;
-    if (texels) *texels = n2;
+    *dptr = map_slot(c, which, slot);
+    if (texels) *texels = (size_t)c->n * c->n;
     return WSO_OK;
 }
 
 int wso_copy_map(wso_ctx* c, int which, uint32_t slot, float* dst) {
+    if (c && c->map_format != WSO_MAP_RGBA32F)
+        return fail(c, WSO_ERR_INVALID_ARG, "wso_copy_map copies RGBA32F maps: use wso_copy_map_bytes");
+    return wso_copy_map_bytes(c, which, slot, dst, c ? map_slot_bytes(c) : 0);
+}
+
+int wso_copy_map_bytes(wso_ctx* c, int which, uint32_t slot, void* dst, size_t dst_bytes) {
     void* src = nullptr;
-    size_t texels = 0;
-    int rc = wso_map_device(c, which, slot, &src, &texels);
+    int rc = wso_map_device(c, which, slot, &src, nullptr);
     if (rc != WSO_OK) return rc;
     if (!dst) return fail(c, WSO_ERR_INVALID_ARG, "dst is NULL");
+    const size_t bytes = map_slot_bytes(c);
+    if (dst_bytes < bytes) return fail(c, WSO_ERR_INVALID_ARG, "dst too small: N*N texels of the map format");
     WSO_CUDA(c, cudaSetDevice(c->device));
-    WSO_CUDA(c, cudaMemcpyAsync(dst, src, sizeof(float4) * texels, cudaMemcpyDeviceToHost, c->stream));
+    WSO_CUDA(c, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
     WSO_CUDA(c, cudaStreamSynchronize(c->stream));
     return WSO_OK;
 }
@@ -1038,7 +1088,7 @@ int wso_set_exportable(wso_ctx* c, int on) {
     if (rc != WSO_OK) return rc;
     const bool before = c->exportable;
     c->exportable = want;
-    const size_t bytes = sizeof(float4) * (size_t)c->n * c->n * c->max_slots;
+    const size_t bytes = map_slot_bytes(c) * c->max_slots;
     for (int which = 0; which < 2; ++which) {
         rc = alloc_map(c, which, bytes);
         if (rc != WSO_OK) {  // fall back to what worked before; the maps must stay usable
@@ -1052,6 +1102,58 @@ int wso_set_exportable(wso_ctx* c, int on) {
     rc = reset_map_contents(c, (size_t)c->n * c->n);
     if (rc != WSO_OK) return rc;
     WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+    return WSO_OK;
+}
+
+// Switch both maps between RGBA32F and RGBA16F: like wso_set_exportable, the map arrays (own or exportable memory; an
+// imported array returns to own memory) and the pinned mirrors are reallocated at the new size and reset to the
+// resize() defaults.  Prepare() state, the tile size and the exportable switch are kept.
+int wso_set_map_format(wso_ctx* c, int format) {
+    if (!c) return WSO_ERR_INVALID_ARG;
+    if (format != WSO_MAP_RGBA32F && format != WSO_MAP_RGBA16F)
+        return fail(c, WSO_ERR_INVALID_ARG, "map format must be WSO_MAP_RGBA32F or WSO_MAP_RGBA16F; unchanged");
+    if (format == c->map_format) return WSO_OK;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    int rc = wso_sync(c);
+    if (rc != WSO_OK) return rc;
+    const int before = c->map_format;
+    c->map_format = format;
+    if (c->n == 0) return WSO_OK;  // no size allocated (a failed size change): the next allocation uses the format
+    const size_t n2 = (size_t)c->n * c->n;
+    auto reallocate = [&]() -> int {
+        cudaFreeHost(c->h_disp); c->h_disp = nullptr;
+        cudaFreeHost(c->h_norm); c->h_norm = nullptr;
+        for (int which = 0; which < 2; ++which) free_map(c, which);
+        WSO_CUDA(c, cudaMallocHost(&c->h_disp, map_texel_bytes(c) * n2));
+        WSO_CUDA(c, cudaMallocHost(&c->h_norm, map_texel_bytes(c) * n2));
+        for (int which = 0; which < 2; ++which) {
+            const int r = alloc_map(c, which, map_slot_bytes(c) * c->max_slots);
+            if (r != WSO_OK) return r;
+        }
+        const int r = reset_map_contents(c, n2);
+        if (r != WSO_OK) return r;
+        WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+        return WSO_OK;
+    };
+    rc = reallocate();
+    if (rc != WSO_OK) {  // fall back to the previous format; the maps must stay usable
+        const std::string msg = c->err;
+        c->map_format = before;
+        if (reallocate() != WSO_OK) {
+            // not even the previous size fits any more: no size is resident (compute calls answer WSO_ERR_NOT_PREPARED)
+            free_device_buffers(c);
+            c->n = 0;
+            c->logn = 0;
+            for (uint32_t t = 0; t < c->max_tiles; ++t) c->tiles[t].is_prepared = false;
+        }
+        return fail(c, rc, msg);
+    }
+    return WSO_OK;
+}
+
+int wso_get_map_format(const wso_ctx* c, int* format) {
+    if (!c || !format) return WSO_ERR_INVALID_ARG;
+    *format = c->map_format;
     return WSO_OK;
 }
 
@@ -1073,7 +1175,7 @@ int wso_export_fd(wso_ctx* c, int which, int* fd, size_t* bytes) {
 int wso_import_external_fd(wso_ctx* c, int which, int fd, size_t bytes, size_t offset) {
     if (!c || fd < 0) return WSO_ERR_INVALID_ARG;
     if (which != WSO_MAP_DISPLACEMENT && which != WSO_MAP_NORMAL) return fail(c, WSO_ERR_INVALID_ARG, "bad map id");
-    const size_t need = sizeof(float4) * (size_t)c->n * c->n * c->max_slots;
+    const size_t need = map_slot_bytes(c) * c->max_slots;
     if (offset % 16 != 0 || offset > bytes || bytes - offset < need)
         return fail(c, WSO_ERR_INVALID_ARG, "external memory too small for max_slots maps at this offset (or offset not 16-byte aligned)");
     WSO_CUDA(c, cudaSetDevice(c->device));

@@ -10,6 +10,7 @@
 #include <string.h>
 
 #if defined(__CUDACC__)
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #define WSO_HD __host__ __device__ __forceinline__
 #else
@@ -93,6 +94,68 @@ WSO_HD void st_stream(float4* p, float4 v) { __stcs(p, v); }
 #else
 WSO_HD void st_stream(float4* p, float4 v) { *p = v; }
 #endif
+
+// ---------------------------------------------------------------------------------------------
+// RGBA16F output texel (wso_set_map_format): (x, y, z, w) as four IEEE binary16 values, little-endian, tightly packed
+// - 8 bytes, VK_FORMAT_R16G16B16A16_SFLOAT.  xy holds x in bits 0..15 and y in bits 16..31, zw likewise.
+// Conversion: the fp32 value the RGBA32F path stores, rounded to nearest even (cvt.rn.f16x2.f32 on the device, one
+// instruction per two channels).  As with any IEEE conversion, magnitudes >= 65520 become +-inf, values below 2^-24
+// go to subnormals / signed zero, and NaN stays NaN.
+// ---------------------------------------------------------------------------------------------
+struct alignas(8) Half4 {
+    uint32_t xy, zw;
+};
+
+#if !defined(__CUDA_ARCH__)
+// Portable float -> binary16 bits, IEEE round to nearest even (the host build of the kernel bodies, tests/emu).
+WSO_HD uint16_t f32_to_f16_rn(float x) {
+    uint32_t u;
+    memcpy(&u, &x, 4);
+    const uint32_t sign = (u >> 16) & 0x8000u;
+    const uint32_t a = u & 0x7fffffffu;
+    if (a > 0x7f800000u) return (uint16_t)(sign | 0x7e00u | ((a >> 13) & 0x3ffu));  // NaN (quiet)
+    if (a >= 0x47800000u) return (uint16_t)(sign | 0x7c00u);                         // >= 2^16 and inf
+    if (a >= 0x38800000u) {
+        // normal binary16 range (>= 2^-14): rebias the exponent by 127 - 15, round the 13 dropped mantissa bits to
+        // nearest even; a carry out of the mantissa steps the exponent (65520 and up -> 0x7c00 = inf)
+        return (uint16_t)(sign | ((a - 0x38000000u + 0xfffu + ((a >> 13) & 1u)) >> 13));
+    }
+    const uint32_t e = a >> 23;
+    if (e < 102u) return (uint16_t)sign;  // below 2^-25: rounds to zero (2^-25 itself is the tie 0 | 2^-24 -> even 0)
+    // subnormal binary16: the value in units of 2^-24 is mant * 2^(e - 126), 14 <= 126 - e <= 24
+    const uint32_t mant = (a & 0x7fffffu) | 0x800000u;
+    const uint32_t s = 126u - e;
+    uint32_t r = mant >> s;
+    const uint32_t rem = mant & ((1u << s) - 1u), half = 1u << (s - 1u);
+    if (rem > half || (rem == half && (r & 1u))) ++r;  // may carry into the smallest normal, 0x0400: still right
+    return (uint16_t)(sign | r);
+}
+#endif
+
+// binary16 bits of (lo, hi) in one 32-bit word, lo in bits 0..15
+#if defined(__CUDA_ARCH__)
+WSO_HD uint32_t half2_bits(float lo, float hi) {
+    const __half2 h = __floats2half2_rn(lo, hi);  // cvt.rn.f16x2.f32
+    uint32_t u;
+    memcpy(&u, &h, 4);
+    return u;
+}
+#else
+WSO_HD uint32_t half2_bits(float lo, float hi) { return (uint32_t)f32_to_f16_rn(lo) | ((uint32_t)f32_to_f16_rn(hi) << 16); }
+#endif
+
+// one 8-byte evict-first store (st.global.cs.v2.b32): same cache policy as the RGBA32F maps
+#if defined(__CUDA_ARCH__) && !defined(WSO_EXP_NO_STREAM_STORES)
+WSO_HD void st_stream(Half4* p, Half4 v) {
+    asm volatile("st.global.cs.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(v.xy), "r"(v.zw) : "memory");
+}
+#else
+WSO_HD void st_stream(Half4* p, Half4 v) { *p = v; }
+#endif
+
+// Store one output texel in the map's format (the kernels compute fp32 either way).
+WSO_HD void st_texel(float4* p, float x, float y, float z, float w) { st_stream(p, make_float4(x, y, z, w)); }
+WSO_HD void st_texel(Half4* p, float x, float y, float z, float w) { st_stream(p, Half4{half2_bits(x, y), half2_bits(z, w)}); }
 // ld_ro: spectrum records are read-only for the lifetime of a launch (experiment hook: the non-coherent path)
 #if defined(__CUDA_ARCH__) && defined(WSO_EXP_LDG_RECORDS)
 WSO_HD float4 ld_ro(const float4* p) { return __ldg(p); }

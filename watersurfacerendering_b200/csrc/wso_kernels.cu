@@ -98,12 +98,13 @@ wso_pass1_kernel(const __grid_constant__ Args args) {
     Pass1<LOGN, TL::CP, TL::NF, false, FAST, JAC>::run(ex, smem, blockIdx.x, blockIdx.y, blockIdx.z, args);
 }
 
-template <int LOGN, class TL, class Args>
+// TEX: output texel of the maps kernels (float4 = RGBA32F, Half4 = RGBA16F; wso_set_map_format)
+template <int LOGN, class TL, class Args, class TEX = float4>
 __global__ void __launch_bounds__(Pass2<LOGN, TL::RI, false>::T, min_blocks(Pass2<LOGN, TL::RI, false>::T))
 wso_pass2_kernel(const __grid_constant__ Args args) {
     extern __shared__ __align__(16) float2 smem[];
     DeviceExec ex;
-    Pass2<LOGN, TL::RI, false>::run(ex, smem, blockIdx.x, blockIdx.y, blockIdx.z, args);
+    Pass2<LOGN, TL::RI, false, false, false, false, TEX>::run(ex, smem, blockIdx.x, blockIdx.y, blockIdx.z, args);
 }
 
 // Persistent forms (Pass1::run_persistent / Pass2::run_persistent): a fixed 1-D grid of CTAs - as many as the device
@@ -135,7 +136,7 @@ wso_pass1p_kernel(const __grid_constant__ Args args, const int n_items) {
     if constexpr (PersistOk<LOGN, TL>::k1)
         Pass1<LOGN, TL::CP, TL::NF, false, true>::run_persistent(ex, smem, blockIdx.x, gridDim.x, n_items, args);
 }
-template <int LOGN, class TL, class Args>
+template <int LOGN, class TL, class Args, class TEX = float4>
 __global__ void __launch_bounds__(Pass2<LOGN, TL::RI, false>::T, min_blocks(Pass2<LOGN, TL::RI, false>::T))
 wso_pass2p_kernel(const __grid_constant__ Args args, const int n_items) {
     extern __shared__ __align__(16) float2 smem[];
@@ -144,7 +145,7 @@ wso_pass2p_kernel(const __grid_constant__ Args args, const int n_items) {
     exp_stagger((blockIdx.x / 148u) * (unsigned)(WSO_EXP_P_STAGGER2_NS));
 #endif
     if constexpr (PersistOk<LOGN, TL>::k2)
-        Pass2<LOGN, TL::RI, false>::run_persistent(ex, smem, blockIdx.x, gridDim.x, n_items, args);
+        Pass2<LOGN, TL::RI, false, false, false, false, TEX>::run_persistent(ex, smem, blockIdx.x, gridDim.x, n_items, args);
 }
 
 // "K2nh": the height pre-pass and the NORMAL map in one launch (blockIdx.y = 0: normal-map CTAs, 1: height CTAs), followed
@@ -160,7 +161,7 @@ struct K2Split {
     static constexpr int SMEM = P2::SMEM_BYTES > PH::SMEM_BYTES ? P2::SMEM_BYTES : PH::SMEM_BYTES;
     static constexpr int GX = P2::H / TL::RI;  // >= the number of height CTAs, H / (2 RI)
 };
-template <int LOGN, class TL, class Args>
+template <int LOGN, class TL, class Args, class TEX = float4>
 __global__ void __launch_bounds__(Pass2<LOGN, TL::RI, false>::T, min_blocks(Pass2<LOGN, TL::RI, false>::T))
 wso_pass2nh_kernel(const __grid_constant__ Args args) {
     extern __shared__ __align__(16) float2 smem[];
@@ -170,7 +171,7 @@ wso_pass2nh_kernel(const __grid_constant__ Args args) {
         // K1 (the predecessor in the stream) must have completed before W is read
         ex.pdl_wait();
         ex.pdl_release();
-        Pass2<LOGN, TL::RI, false>::run(ex, smem, blockIdx.x, 1, blockIdx.z, args);
+        Pass2<LOGN, TL::RI, false, false, false, false, TEX>::run(ex, smem, blockIdx.x, 1, blockIdx.z, args);
     } else {
         using PH = typename K2Split<LOGN, TL>::PH;
         if (blockIdx.x >= PH::grid_x()) return;
@@ -181,12 +182,12 @@ wso_pass2nh_kernel(const __grid_constant__ Args args) {
 // K2 with the Jacobian channel: one row item (all four packed fields) per CTA, both maps from one CTA.
 // Sizes up to 4096^2 (four lines of shared memory and 4*N/16 <= 1024 threads).
 constexpr bool jacobian_size_ok(int logn) { return logn <= 12; }
-template <int LOGN, class Args>
+template <int LOGN, class Args, class TEX = float4>
 __global__ void __launch_bounds__(Pass2<LOGN, 1, false, false, false, true>::T)
 wso_pass2j_kernel(const __grid_constant__ Args args) {
     extern __shared__ __align__(16) float2 smem[];
     DeviceExec ex;
-    Pass2<LOGN, 1, false, false, false, true>::run(ex, smem, blockIdx.x, 0, blockIdx.z, args);
+    Pass2<LOGN, 1, false, false, false, true, TEX>::run(ex, smem, blockIdx.x, 0, blockIdx.z, args);
 }
 
 // K2h: height extrema (min/max -> amplitude A) ahead of K2, so that K2 writes disp.y already normalised and no
@@ -281,7 +282,7 @@ static int resident_ctas(Kern kern, int threads, int smem, int dev) {
 }
 
 // Jacobian mode: K1 (general body, field 1 with its real slot filled), K2h, K2 with four lines per CTA
-template <int LOGN, class TL, class Args>
+template <int LOGN, class TL, class Args, class TEX>
 static cudaError_t launch_tiled_jacobian(const Args& args, int n_items, cudaStream_t stream, cudaEvent_t* ev) {
     if constexpr (!jacobian_size_ok(LOGN)) {
         return cudaErrorNotSupported;
@@ -296,7 +297,7 @@ static cudaError_t launch_tiled_jacobian(const Args& args, int n_items, cudaStre
         if (dev < 0 || dev >= 16 || !configured[dev].load(std::memory_order_acquire)) {
             e = cudaFuncSetAttribute(wso_pass1_kernel<LOGN, TL, Args, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, P1::SMEM_BYTES);
             if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(wso_pass2j_kernel<LOGN, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, PJ::SMEM_BYTES);
+            e = cudaFuncSetAttribute(wso_pass2j_kernel<LOGN, Args, TEX>, cudaFuncAttributeMaxDynamicSharedMemorySize, PJ::SMEM_BYTES);
             if (e != cudaSuccess) return e;
             e = cudaFuncSetAttribute(wso_heights_kernel<LOGN, TL, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH::SMEM_BYTES);
             if (e != cudaSuccess) return e;
@@ -311,7 +312,7 @@ static cudaError_t launch_tiled_jacobian(const Args& args, int n_items, cudaStre
         e = launch_pdl(wso_heights_kernel<LOGN, TL, Args>, dim3(PH::grid_x(), 1, n_items), PH::T, PH::SMEM_BYTES, stream, args);
         if (e != cudaSuccess) return e;
         if (ev) cudaEventRecord(ev[2], stream);
-        e = launch_pdl(wso_pass2j_kernel<LOGN, Args>, dim3(PJ::H, 1, n_items), PJ::T, PJ::SMEM_BYTES, stream, args);
+        e = launch_pdl(wso_pass2j_kernel<LOGN, Args, TEX>, dim3(PJ::H, 1, n_items), PJ::T, PJ::SMEM_BYTES, stream, args);
         if (e != cudaSuccess) return e;
         if (ev) cudaEventRecord(ev[3], stream);
         return cudaGetLastError();
@@ -342,7 +343,7 @@ static int exp_min_smem(const char* name) {
     return v > 0 && v <= 227 * 1024 ? v : 0;
 }
 
-template <int LOGN, class TL, class Args>
+template <int LOGN, class TL, class Args, class TEX>
 static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stream, cudaEvent_t* ev) {
     using P1 = Pass1<LOGN, TL::CP, TL::NF>;
     using P2 = Pass2<LOGN, TL::RI, false>;
@@ -362,7 +363,7 @@ static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stre
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(wso_pass1_kernel<LOGN, TL, Args, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem1);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wso_pass2_kernel<LOGN, TL, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2);
+        e = cudaFuncSetAttribute(wso_pass2_kernel<LOGN, TL, Args, TEX>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2);
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(wso_heights_kernel<LOGN, TL, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH::SMEM_BYTES);
         if (e != cudaSuccess) return e;
@@ -373,14 +374,14 @@ static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stre
                 if (dev >= 0 && dev < 16) ctas1[dev] = resident_ctas(wso_pass1p_kernel<LOGN, TL, Args>, P1::T, P1::SMEM_BYTES, dev);
             }
             if constexpr (PersistOk<LOGN, TL>::k2) {
-                e = cudaFuncSetAttribute(wso_pass2p_kernel<LOGN, TL, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2::SMEM_BYTES);
+                e = cudaFuncSetAttribute(wso_pass2p_kernel<LOGN, TL, Args, TEX>, cudaFuncAttributeMaxDynamicSharedMemorySize, P2::SMEM_BYTES);
                 if (e != cudaSuccess) return e;
-                if (dev >= 0 && dev < 16) ctas2[dev] = resident_ctas(wso_pass2p_kernel<LOGN, TL, Args>, P2::T, P2::SMEM_BYTES, dev);
+                if (dev >= 0 && dev < 16) ctas2[dev] = resident_ctas(wso_pass2p_kernel<LOGN, TL, Args, TEX>, P2::T, P2::SMEM_BYTES, dev);
             }
         }
         if constexpr (K2Split<LOGN, TL>::possible) {
             const int smemnh = K2Split<LOGN, TL>::SMEM > k2_min ? K2Split<LOGN, TL>::SMEM : k2_min;
-            e = cudaFuncSetAttribute(wso_pass2nh_kernel<LOGN, TL, Args>, cudaFuncAttributeMaxDynamicSharedMemorySize, smemnh);
+            e = cudaFuncSetAttribute(wso_pass2nh_kernel<LOGN, TL, Args, TEX>, cudaFuncAttributeMaxDynamicSharedMemorySize, smemnh);
             if (e != cudaSuccess) return e;
         }
         if (dev >= 0 && dev < 16) configured[dev].store(true, std::memory_order_release);
@@ -399,6 +400,8 @@ static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stre
     if constexpr (std::is_same<Args, LaunchArgs>::value) {
         if (fast && warp_core_supported(LOGN)) warp_mask = warp_core_mask(LOGN);
     }
+    // the warp-per-line K2 writes RGBA32F only: RGBA16F maps always come from the CTA-per-line K2 (bit 2 ignored)
+    if constexpr (!std::is_same<TEX, float4>::value) warp_mask &= ~4;
     if constexpr (std::is_same<Args, LaunchArgs>::value) {
         if (warp_mask & 1) e = launch_warp_core(LOGN, 0, args, n_items, stream);
     }
@@ -424,10 +427,10 @@ static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stre
         if (!(warp_mask & 6) && k2_split_enabled()) {
             using KS = K2Split<LOGN, TL>;
             const int smemnh = KS::SMEM > k2_min ? KS::SMEM : k2_min;
-            e = launch_pdl(wso_pass2nh_kernel<LOGN, TL, Args>, dim3(KS::GX, 2, n_items), P2::T, smemnh, stream, args);
+            e = launch_pdl(wso_pass2nh_kernel<LOGN, TL, Args, TEX>, dim3(KS::GX, 2, n_items), P2::T, smemnh, stream, args);
             if (e != cudaSuccess) return e;
             if (ev) cudaEventRecord(ev[2], stream);
-            e = launch_pdl(wso_pass2_kernel<LOGN, TL, Args>, dim3(P2::H / TL::RI, 1, n_items), P2::T, smem2, stream, args);
+            e = launch_pdl(wso_pass2_kernel<LOGN, TL, Args, TEX>, dim3(P2::H / TL::RI, 1, n_items), P2::T, smem2, stream, args);
             if (e != cudaSuccess) return e;
             if (ev) cudaEventRecord(ev[3], stream);
             return cudaGetLastError();
@@ -449,21 +452,21 @@ static cudaError_t launch_tiled(const Args& args, int n_items, cudaStream_t stre
         if (!k2_done && (persist & 4)) {
             const int total = (int)(g2.x * g2.y * g2.z);
             const int grid = total < ctas2[dev] ? total : ctas2[dev];
-            e = launch_pdl(wso_pass2p_kernel<LOGN, TL, Args>, dim3(grid, 1, 1), P2::T, P2::SMEM_BYTES, stream, args, n_items);
+            e = launch_pdl(wso_pass2p_kernel<LOGN, TL, Args, TEX>, dim3(grid, 1, 1), P2::T, P2::SMEM_BYTES, stream, args, n_items);
             k2_done = true;
         }
     }
-    if (!k2_done) e = launch_pdl(wso_pass2_kernel<LOGN, TL, Args>, g2, P2::T, smem2, stream, args);
+    if (!k2_done) e = launch_pdl(wso_pass2_kernel<LOGN, TL, Args, TEX>, g2, P2::T, smem2, stream, args);
     if (e != cudaSuccess) return e;
     if (ev) cudaEventRecord(ev[3], stream);
     return cudaGetLastError();
 }
 
-template <int LOGN>
+template <int LOGN, class TEX>
 static cudaError_t launch_all(const LaunchArgs& args, int n_items, cudaStream_t stream, bool jacobian, cudaEvent_t* ev) {
     using B = typename Cfg<LOGN>::Bulk;
     using L = typename Cfg<LOGN>::Lat;
-    if (jacobian) return launch_tiled_jacobian<LOGN, B, LaunchArgs>(args, n_items, stream, ev);
+    if (jacobian) return launch_tiled_jacobian<LOGN, B, LaunchArgs, TEX>(args, n_items, stream, ev);
     // few tile-frames in this launch: the Bulk grid of K1 would leave SMs idle -> fine-grained tiling and the
     // small parameter block
     constexpr int bulk_ctas_per_item = ((1 << LOGN) / 2 / B::CP) * (4 / B::NF);
@@ -472,28 +475,34 @@ static cudaError_t launch_all(const LaunchArgs& args, int n_items, cudaStream_t 
         sm.tw = args.tw; sm.W = args.W; sm.disp = args.disp; sm.norm = args.norm;
         sm.minmax = args.minmax; sm.amp_out = args.amp_out;
         for (int i = 0; i < kSmallChunk; ++i) { sm.items[i] = args.items[i]; sm.td[i] = args.td[i]; }
-        return launch_tiled<LOGN, L, LaunchArgsSmall>(sm, n_items, stream, ev);
+        return launch_tiled<LOGN, L, LaunchArgsSmall, TEX>(sm, n_items, stream, ev);
     }
-    return launch_tiled<LOGN, B, LaunchArgs>(args, n_items, stream, ev);
+    return launch_tiled<LOGN, B, LaunchArgs, TEX>(args, n_items, stream, ev);
+}
+template <int LOGN>
+static cudaError_t launch_all(const LaunchArgs& args, int n_items, cudaStream_t stream, bool jacobian, bool half,
+                              cudaEvent_t* ev) {
+    return half ? launch_all<LOGN, Half4>(args, n_items, stream, jacobian, ev)
+                : launch_all<LOGN, float4>(args, n_items, stream, jacobian, ev);
 }
 
 cudaError_t launch_compute_waves(int logn, const LaunchArgs& args, int n_items, cudaStream_t stream,
-                                 bool jacobian, cudaEvent_t* ev) {
+                                 bool jacobian, bool half, cudaEvent_t* ev) {
     switch (logn) {
 // WSO_ONLY_LOGN: tuning builds instantiate a single size (tools/tune_build.sh) to keep compile times short
 #ifdef WSO_ONLY_LOGN
-        case WSO_ONLY_LOGN: return launch_all<WSO_ONLY_LOGN>(args, n_items, stream, jacobian, ev);
+        case WSO_ONLY_LOGN: return launch_all<WSO_ONLY_LOGN>(args, n_items, stream, jacobian, half, ev);
 #else
-        case 4: return launch_all<4>(args, n_items, stream, jacobian, ev);
-        case 5: return launch_all<5>(args, n_items, stream, jacobian, ev);
-        case 6: return launch_all<6>(args, n_items, stream, jacobian, ev);
-        case 7: return launch_all<7>(args, n_items, stream, jacobian, ev);
-        case 8: return launch_all<8>(args, n_items, stream, jacobian, ev);
-        case 9: return launch_all<9>(args, n_items, stream, jacobian, ev);
-        case 10: return launch_all<10>(args, n_items, stream, jacobian, ev);
-        case 11: return launch_all<11>(args, n_items, stream, jacobian, ev);
-        case 12: return launch_all<12>(args, n_items, stream, jacobian, ev);
-        case 13: return launch_all<13>(args, n_items, stream, jacobian, ev);
+        case 4: return launch_all<4>(args, n_items, stream, jacobian, half, ev);
+        case 5: return launch_all<5>(args, n_items, stream, jacobian, half, ev);
+        case 6: return launch_all<6>(args, n_items, stream, jacobian, half, ev);
+        case 7: return launch_all<7>(args, n_items, stream, jacobian, half, ev);
+        case 8: return launch_all<8>(args, n_items, stream, jacobian, half, ev);
+        case 9: return launch_all<9>(args, n_items, stream, jacobian, half, ev);
+        case 10: return launch_all<10>(args, n_items, stream, jacobian, half, ev);
+        case 11: return launch_all<11>(args, n_items, stream, jacobian, half, ev);
+        case 12: return launch_all<12>(args, n_items, stream, jacobian, half, ev);
+        case 13: return launch_all<13>(args, n_items, stream, jacobian, half, ev);
 #endif
         default: return cudaErrorInvalidValue;
     }
@@ -507,17 +516,18 @@ void destroy_frame_graph(FrameGraph& g) {
     g.exec = nullptr;
     g.graph = nullptr;
     g.n_nodes = 0;
-    g.logn = g.jacobian = -1;
+    g.logn = g.jacobian = g.half = -1;
 }
 
 // Capture the launch sequence of one tile-frame into g (stream must not be capturing already).  false: not capturable here.
-static bool capture_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian) {
+static bool capture_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian,
+                                bool half) {
     destroy_frame_graph(g);
     if (cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
         cudaGetLastError();
         return false;
     }
-    const cudaError_t le = launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+    const cudaError_t le = launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
     cudaGraph_t graph = nullptr;
     const cudaError_t ce = cudaStreamEndCapture(stream, &graph);
     bool ok = le == cudaSuccess && ce == cudaSuccess && graph != nullptr;
@@ -543,37 +553,40 @@ static bool capture_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args,
     g.n_nodes = (int)n;
     g.logn = logn;
     g.jacobian = jacobian ? 1 : 0;
+    g.half = half ? 1 : 0;
     g.captures += 1;
     return true;
 }
 
-cudaError_t launch_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian) {
+cudaError_t launch_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian,
+                               bool half) {
     // kernels of wso_kernels2.cu (an explicit kernel-set choice) launch through their own helper: plain launches
-    if (g.disabled || (kernel_choice_mask(logn) & 7) != 0) return launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+    if (g.disabled || (kernel_choice_mask(logn) & 7) != 0) return launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
     // a caller that is capturing this stream into a graph of its own gets the three kernels recorded as they are
     cudaStreamCaptureStatus capturing = cudaStreamCaptureStatusNone;
     if (cudaStreamIsCapturing(stream, &capturing) != cudaSuccess || capturing != cudaStreamCaptureStatusNone) {
         cudaGetLastError();
-        return launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+        return launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
     }
-    if (g.warm_logn != logn || g.warm_jacobian != (jacobian ? 1 : 0)) {
+    if (g.warm_logn != logn || g.warm_jacobian != (jacobian ? 1 : 0) || g.warm_half != (half ? 1 : 0)) {
         // first frame of this shape: the plain launch also does the one-time kernel configuration (cudaFuncSetAttribute)
-        const cudaError_t e = launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+        const cudaError_t e = launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
         if (e == cudaSuccess) {
             g.warm_logn = logn;
             g.warm_jacobian = jacobian ? 1 : 0;
+            g.warm_half = half ? 1 : 0;
         }
         return e;
     }
     for (int attempt = 0; attempt < 2; ++attempt) {
-        if (!g.exec || g.logn != logn || g.jacobian != (jacobian ? 1 : 0)) {
-            if (!capture_frame_graph(g, logn, args, stream, jacobian)) break;
+        if (!g.exec || g.logn != logn || g.jacobian != (jacobian ? 1 : 0) || g.half != (half ? 1 : 0)) {
+            if (!capture_frame_graph(g, logn, args, stream, jacobian, half)) break;
             g.graph_launches += 1;
             return cudaGraphLaunch(g.exec, stream);  // captured with this call's parameters
         }
         GraphUpdate u{&g, 0u, false};
         tl_graph_update = &u;
-        const cudaError_t e = launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+        const cudaError_t e = launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
         tl_graph_update = nullptr;
         if (e == cudaSuccess && !u.mismatch && u.used == (1u << g.n_nodes) - 1u) {
             g.graph_launches += 1;
@@ -584,7 +597,7 @@ cudaError_t launch_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, 
     }
     g.disabled = true;
     destroy_frame_graph(g);
-    return launch_compute_waves(logn, args, 1, stream, jacobian, nullptr);
+    return launch_compute_waves(logn, args, 1, stream, jacobian, half, nullptr);
 }
 
 }  // namespace wso

@@ -3,7 +3,7 @@
 //   K1  Pass1  : spectrum evolve h0 -> h~(k,t) -> 4 real packed spectra Z_f, fused with the first 1-D
 //                transform (along m, two real columns per complex FFT) -> Hermitian half W[m'][f][slot]
 //   K2  Pass2  : second 1-D transform (along n) fused with sign fix, lambda and packing into the
-//                RGBA32F displacement / normal maps + height min/max
+//                RGBA32F (or, opt-in, RGBA16F) displacement / normal maps + height min/max
 //   K3  Normalize : disp.y *= 1/A,  A = max(|min|,|max|)       (reference: WSTessendorf.cpp:443-455)
 //
 // Replaces reference WSTessendorf::ComputeWaves (src/scene/WSTessendorf.cpp:284-441) including the
@@ -11,6 +11,7 @@
 #pragma once
 
 #include <cstring>
+#include <type_traits>
 
 #include "wso_device.cuh"
 
@@ -74,7 +75,7 @@ struct LaunchArgsT {
     static constexpr int kCap = CAP;
     const float2* tw;      // [N] exp(+2*pi*i*k/N)
     float2* W;             // chunk scratch: [item][N/2][4][N]
-    float4* disp;          // [slot][N*N]
+    float4* disp;          // [slot][N*N]  (RGBA16F maps: the K2 instantiations with TEX = Half4 read it as Half4*)
     float4* norm;          // [slot][N*N]
     float* minmax;         // [slot][2]
     float* amp_out;        // [slot] amplitude A
@@ -934,7 +935,9 @@ WSO_HD float amplitude_of(float mn, float mx) {
 //        its partner's line through distributed shared memory.
 // JAC  : SURVEY row f-4 (reference COMPUTE_JACOBIAN, WSTessendorf.cpp:421-428): one CTA transforms all FOUR packed
 //        fields of a row item (by = 0 only) and writes both maps, disp.w = the Jacobian of the horizontal displacement.
-template <int LOGN, int RI, bool HEIGHT_ONLY, bool SLAB = false, bool PAIR = false, bool JAC = false>
+// TEX  : output texel, float4 (RGBA32F) or Half4 (RGBA16F, wso_device.cuh): LaunchArgsT::disp / norm are read as arrays
+//        of TEX.  The arithmetic is the same; only the final store converts.  Single-device kernels only.
+template <int LOGN, int RI, bool HEIGHT_ONLY, bool SLAB = false, bool PAIR = false, bool JAC = false, class TEX = float4>
 struct Pass2 {
     static constexpr int N = 1 << LOGN;
     static constexpr int H = N / 2;
@@ -950,6 +953,8 @@ struct Pass2 {
     static_assert(H % RI == 0, "bad tiling");
     static_assert(!PAIR || (!HEIGHT_ONLY && RI == 1), "cluster pairs: one row item per CTA pair");
     static_assert(!JAC || (!HEIGHT_ONLY && !SLAB && !PAIR), "Jacobian variant: single-device maps kernel only");
+    static_assert(std::is_same<TEX, float4>::value || (std::is_same<TEX, Half4>::value && !SLAB && !PAIR),
+                  "RGBA16F maps: single-device kernels only");
 
     template <class Args>
     static WSO_HD int hl_log(const Args& args) { return SLAB ? LOGN - 1 - args.slab_shift : LOGN - 1; }
@@ -1257,7 +1262,7 @@ struct Pass2 {
 #endif
     static constexpr int kPackUnroll = WSO_TUNE_PACK_UNROLL;
     template <int STRIDE>
-    static WSO_HD void pack_item(const float2* l0, const float2* l1, int mp, float4* outA, float4* outB, int by,
+    static WSO_HD void pack_item(const float2* l0, const float2* l1, int mp, TEX* outA, TEX* outB, int by,
                                  float lambda, float inv_amp, int lt, int rows) {
         static_assert(N % STRIDE == 0, "bad pack stride");
         constexpr int VISITS = N / STRIDE;
@@ -1274,8 +1279,8 @@ struct Pass2 {
                     const int cm = (N - c) & (N - 1);   // row N-m' is the conjugate mirror of row m'
                     const float y = rmul(rmul(a0.x, s), inv_amp);
                     const float x = rmul(sl, a0.y), z = rmul(sl, a1.y);
-                    if (rows & 1) st_stream(&outA[c], make_float4(x, y, z, 1.0f));
-                    if (rows & 2) st_stream(&outB[cm], make_float4(-x, y, -z, 1.0f));
+                    if (rows & 1) st_texel(&outA[c], x, y, z, 1.0f);
+                    if (rows & 2) st_texel(&outB[cm], -x, y, -z, 1.0f);
                 }
             } else {
 #pragma unroll kPackUnroll
@@ -1285,8 +1290,8 @@ struct Pass2 {
                     const float2 a0 = l0[e], a1 = l1[e];
                     const int cm = (N - c) & (N - 1);
                     const float4 ta = make_float4(s * a0.y, s * a1.y, s * a0.x, s * a1.x);
-                    if (rows & 1) st_stream(&outA[c], ta);
-                    if (rows & 2) st_stream(&outB[cm], make_float4(-ta.x, -ta.y, ta.z, ta.w));
+                    if (rows & 1) st_texel(&outA[c], ta.x, ta.y, ta.z, ta.w);
+                    if (rows & 2) st_texel(&outB[cm], -ta.x, -ta.y, ta.z, ta.w);
                 }
             }
         } else {
@@ -1299,11 +1304,11 @@ struct Pass2 {
                 const float2 b0 = make_float2(0.5f * (p0.y + m0.y), -0.5f * (p0.x - m0.x));
                 const float2 b1 = make_float2(0.5f * (p1.y + m1.y), -0.5f * (p1.x - m1.x));
                 if (by == 0) {
-                    if (rows & 1) st_stream(&outA[c], make_float4(rmul(sl, a0.y), rmul(rmul(a0.x, s), inv_amp), rmul(sl, a1.y), 1.0f));
-                    if (rows & 2) st_stream(&outB[c], make_float4(rmul(sl, b0.y), rmul(rmul(b0.x, s), inv_amp), rmul(sl, b1.y), 1.0f));
+                    if (rows & 1) st_texel(&outA[c], rmul(sl, a0.y), rmul(rmul(a0.x, s), inv_amp), rmul(sl, a1.y), 1.0f);
+                    if (rows & 2) st_texel(&outB[c], rmul(sl, b0.y), rmul(rmul(b0.x, s), inv_amp), rmul(sl, b1.y), 1.0f);
                 } else {
-                    if (rows & 1) st_stream(&outA[c], make_float4(s * a0.y, s * a1.y, s * a0.x, s * a1.x));
-                    if (rows & 2) st_stream(&outB[c], make_float4(s * b0.y, s * b1.y, s * b0.x, s * b1.x));
+                    if (rows & 1) st_texel(&outA[c], s * a0.y, s * a1.y, s * a0.x, s * a1.x);
+                    if (rows & 2) st_texel(&outB[c], s * b0.y, s * b1.y, s * b0.x, s * b1.x);
                 }
             }
         }
@@ -1317,7 +1322,7 @@ struct Pass2 {
     }
     template <int STRIDE>
     static WSO_HD void pack_item_jac(const float2* l0, const float2* l1, const float2* l2, const float2* l3, int mp,
-                                     float4* dA, float4* dB, float4* nA, float4* nB, float lambda, float inv_amp,
+                                     TEX* dA, TEX* dB, TEX* nA, TEX* nB, float lambda, float inv_amp,
                                      int lt) {
         const float s = ((mp + lt) & 1) ? -1.0f : 1.0f;
         const float sl = rmul(s, lambda);
@@ -1329,11 +1334,11 @@ struct Pass2 {
                 const float y = rmul(rmul(a0.x, s), inv_amp);
                 const float x = rmul(sl, a0.y), z = rmul(sl, a1.y);
                 const float j = jacobian_of(lambda, s * a2.x, s * a3.x, s * a1.x);
-                st_stream(&dA[c], make_float4(x, y, z, j));
-                st_stream(&dB[cm], make_float4(-x, y, -z, j));
+                st_texel(&dA[c], x, y, z, j);
+                st_texel(&dB[cm], -x, y, -z, j);
                 const float4 ta = make_float4(s * a2.y, s * a3.y, s * a2.x, s * a3.x);
-                st_stream(&nA[c], ta);
-                st_stream(&nB[cm], make_float4(-ta.x, -ta.y, ta.z, ta.w));
+                st_texel(&nA[c], ta.x, ta.y, ta.z, ta.w);
+                st_texel(&nB[cm], -ta.x, -ta.y, ta.z, ta.w);
             }
         } else {
             // rows 0 and N/2 were transformed as one complex line per field: separate them
@@ -1347,12 +1352,12 @@ struct Pass2 {
                     a[f] = make_float2(0.5f * (p.x + m.x), 0.5f * (p.y - m.y));
                     b[f] = make_float2(0.5f * (p.y + m.y), -0.5f * (p.x - m.x));
                 }
-                st_stream(&dA[c], make_float4(rmul(sl, a[0].y), rmul(rmul(a[0].x, s), inv_amp), rmul(sl, a[1].y),
-                                              jacobian_of(lambda, s * a[2].x, s * a[3].x, s * a[1].x)));
-                st_stream(&dB[c], make_float4(rmul(sl, b[0].y), rmul(rmul(b[0].x, s), inv_amp), rmul(sl, b[1].y),
-                                              jacobian_of(lambda, s * b[2].x, s * b[3].x, s * b[1].x)));
-                st_stream(&nA[c], make_float4(s * a[2].y, s * a[3].y, s * a[2].x, s * a[3].x));
-                st_stream(&nB[c], make_float4(s * b[2].y, s * b[3].y, s * b[2].x, s * b[3].x));
+                st_texel(&dA[c], rmul(sl, a[0].y), rmul(rmul(a[0].x, s), inv_amp), rmul(sl, a[1].y),
+                         jacobian_of(lambda, s * a[2].x, s * a[3].x, s * a[1].x));
+                st_texel(&dB[c], rmul(sl, b[0].y), rmul(rmul(b[0].x, s), inv_amp), rmul(sl, b[1].y),
+                         jacobian_of(lambda, s * b[2].x, s * b[3].x, s * b[1].x));
+                st_texel(&nA[c], s * a[2].y, s * a[3].y, s * a[2].x, s * a[3].x);
+                st_texel(&nB[c], s * b[2].y, s * b[3].y, s * b[2].x, s * b[3].x);
             }
         }
     }
@@ -1385,8 +1390,8 @@ struct Pass2 {
         const int hlog = hl_log(args);
         const size_t rows_per_slot = SLAB ? ((size_t)2 << hlog) : (size_t)N;
         if constexpr (JAC) {
-            float4* outd = args.disp + (size_t)item.slot * ((size_t)N * N);
-            float4* outn = args.norm + (size_t)item.slot * ((size_t)N * N);
+            TEX* outd = reinterpret_cast<TEX*>(args.disp) + (size_t)item.slot * ((size_t)N * N);
+            TEX* outn = reinterpret_cast<TEX*>(args.norm) + (size_t)item.slot * ((size_t)N * N);
             ex.each([&](int tid, ThreadState&) {
                 const int ri = tid / GI, lt = tid % GI;
                 const int mp = bx * RI + ri;
@@ -1397,7 +1402,7 @@ struct Pass2 {
             });
             return;
         }
-        float4* out = (by == 0 ? args.disp : args.norm) + (size_t)item.slot * (rows_per_slot * N);
+        TEX* out = reinterpret_cast<TEX*>(by == 0 ? args.disp : args.norm) + (size_t)item.slot * (rows_per_slot * N);
         ex.each([&](int tid, ThreadState&) {
             const int ri = tid / GI, lt = tid % GI;
             const int ml = bx * RI + ri;
@@ -1412,8 +1417,8 @@ struct Pass2 {
                 l0 = smem + (ri * 2 + 0) * LS;
                 l1 = l0 + LS;
             }
-            float4* outA = out + (size_t)(SLAB ? ml : mp) * N;
-            float4* outB = out + (size_t)(SLAB ? (1 << hlog) + ml : (mp == 0 ? H : N - mp)) * N;
+            TEX* outA = out + (size_t)(SLAB ? ml : mp) * N;
+            TEX* outB = out + (size_t)(SLAB ? (1 << hlog) + ml : (mp == 0 ? H : N - mp)) * N;
             pack_item<GI>(l0, l1, mp, outA, outB, by, lambda, inv_amp, lt, rows);
         });
     }
@@ -1469,12 +1474,12 @@ struct Pass2 {
                 if (tid == 0) args.amp_out[item.slot] = amp;
             });
         }
-        float4* out = (by == 0 ? args.disp : args.norm) + (size_t)item.slot * ((size_t)N * N);
+        TEX* out = reinterpret_cast<TEX*>(by == 0 ? args.disp : args.norm) + (size_t)item.slot * ((size_t)N * N);
         ex.each([&](int tid, ThreadState& st) {
             const int line = tid / G, j = tid % G;
             const int mp = bx * RI + line / 2;
-            float4* outA = out + (size_t)mp * N;
-            float4* outB = out + (size_t)(mp == 0 ? H : N - mp) * N;
+            TEX* outA = out + (size_t)mp * N;
+            TEX* outB = out + (size_t)(mp == 0 ? H : N - mp) * N;
             if (mp == 0) {
                 const float2* l0 = smem + (line & ~1) * LS;
                 pack_item<GI>(l0, l0 + LS, mp, outA, outB, by, lambda, inv_amp, tid % GI, 3);
@@ -1489,12 +1494,12 @@ struct Pass2 {
                 if (by == 0) {
                     const float y = rmul(rmul(a0.x, s), inv_amp);
                     const float x = rmul(sl, a0.y), z = rmul(sl, a1.y);
-                    st_stream(&outA[c], make_float4(x, y, z, 1.0f));
-                    st_stream(&outB[cm], make_float4(-x, y, -z, 1.0f));
+                    st_texel(&outA[c], x, y, z, 1.0f);
+                    st_texel(&outB[cm], -x, y, -z, 1.0f);
                 } else {
                     const float4 ta = make_float4(s * a0.y, s * a1.y, s * a0.x, s * a1.x);
-                    st_stream(&outA[c], ta);
-                    st_stream(&outB[cm], make_float4(-ta.x, -ta.y, ta.z, ta.w));
+                    st_texel(&outA[c], ta.x, ta.y, ta.z, ta.w);
+                    st_texel(&outB[cm], -ta.x, -ta.y, ta.z, ta.w);
                 }
             };
             if ((line & 1) == 0) {  // this thread holds packed field 0 (or 2): columns r < HALF

@@ -17,14 +17,16 @@ static constexpr int kMaxLogN = 13;  // 8192 (single-CTA line transforms; larger
 // ev: NULL, or 4 events recorded before K1, between the kernels and after K2 (opt-in profiling).
 // jacobian: write disp.w = Jacobian of the horizontal displacement (SURVEY row f-4; sizes up to 4096^2, else
 // cudaErrorNotSupported) instead of the reference default 1.0f.
+// half: K2 writes RGBA16F texels (8 bytes, wso_device.cuh Half4) into args.disp / args.norm, slot stride 8*N*N bytes,
+// instead of RGBA32F (always through the CTA-per-line K2, whatever the kernel-set mask says for K2).
 cudaError_t launch_compute_waves(int logn, const LaunchArgs& args, int n_items, cudaStream_t stream,
-                                 bool jacobian, cudaEvent_t* ev);
+                                 bool jacobian, bool half, cudaEvent_t* ev);
 static constexpr int kMaxJacobianLogN = 12;
 int kernels_per_launch();
 
 // One tile-frame as a CUDA graph (the reference's calling pattern: one ComputeWaves(t) per rendered frame).  The three
 // launches of a frame cost ~13 us of host enqueue through the runtime - more than the kernels take on the device at 512^2 -
-// so a context keeps the launch sequence of its current (size, jacobian) as an instantiated graph (captured from the very
+// so a context keeps the launch sequence of its current (size, jacobian, map format) as an instantiated graph (captured from the very
 // same launch code, programmatic-dependent-launch edges included), rewrites the kernel parameters of its nodes per call
 // (cudaGraphExecKernelNodeSetParams) and pays one cudaGraphLaunch.
 struct FrameGraph {
@@ -34,13 +36,14 @@ struct FrameGraph {
     cudaGraphNode_t node[kMaxNodes] = {};
     void* func[kMaxNodes] = {};
     int n_nodes = 0;
-    int logn = -1, jacobian = -1;            // what the instantiated graph was captured for
-    int warm_logn = -1, warm_jacobian = -1;  // a plain launch of this shape has run (one-time kernel configuration done)
+    int logn = -1, jacobian = -1, half = -1;                  // what the instantiated graph was captured for
+    int warm_logn = -1, warm_jacobian = -1, warm_half = -1;  // a plain launch of this shape has run (one-time kernel configuration done)
     bool disabled = false;                   // capture or instantiation failed once: plain launches from then on
     uint64_t graph_launches = 0, captures = 0;
 };
 // args.items[0] = the tile-frame.  Falls back to launch_compute_waves whenever the graph cannot be used.
-cudaError_t launch_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian);
+cudaError_t launch_frame_graph(FrameGraph& g, int logn, const LaunchArgs& args, cudaStream_t stream, bool jacobian,
+                               bool half);
 void destroy_frame_graph(FrameGraph& g);
 
 // Warp-per-line kernels (wso_kernels2.cu): 512^2, 1024^2 and 2048^2, every item with the sincos table and the pair-summed

@@ -80,6 +80,7 @@ class WSTessendorf:
         self.max_slots = int(max_slots)
         self._min = np.float32(-1.0)   # reference: WSTessendorf.h:226-227
         self._max = np.float32(1.0)
+        self._map_dtype = np.float32   # texel channel type of both maps (set_map_format)
 
     # ------------------------------------------------------------------ lifetime
     def close(self):
@@ -218,16 +219,38 @@ class WSTessendorf:
         return np.float32(a.value)
 
     def _host_map(self, which) -> np.ndarray:
+        n = self.GetTileSize()
+        if self._map_dtype is np.float16:
+            p, nbytes = C.c_void_p(), C.c_size_t()
+            L.check(self._lib.wso_map_host_bytes(self._h, which, C.byref(p), C.byref(nbytes)), self._h)
+            buf = (C.c_char * nbytes.value).from_address(p.value)
+            return np.frombuffer(buf, dtype=np.float16).reshape(n, n, 4)
         p, cnt = C.c_void_p(), C.c_size_t()
         L.check(self._lib.wso_map_host(self._h, which, C.byref(p), C.byref(cnt)), self._h)
-        n = self.GetTileSize()
         buf = (C.c_float * (cnt.value * 4)).from_address(p.value)
         return np.frombuffer(buf, dtype=np.float32).reshape(n, n, 4)
+
+    # ---- map format (extension: RGBA16F maps, half the bytes of the reference's RGBA32F)
+    def set_map_format(self, fmt: str):
+        """"rgba32f" (default, the reference's format) or "rgba16f": 4 x binary16 per texel, each channel the fp32 value
+        rounded to nearest even.  Reallocates the maps (contents reset to the resize() defaults); Prepare() state is kept.
+        In "rgba16f" the map accessors return np.float16 arrays."""
+        code = {"rgba32f": L.WSO_MAP_RGBA32F, "rgba16f": L.WSO_MAP_RGBA16F}.get(fmt)
+        if code is None:
+            raise ValueError(f"map format must be 'rgba32f' or 'rgba16f', not {fmt!r}")
+        L.check(self._lib.wso_set_map_format(self._h, code), self._h)
+        self._map_dtype = np.float16 if code == L.WSO_MAP_RGBA16F else np.float32
+
+    def get_map_format(self) -> str:
+        v = C.c_int()
+        L.check(self._lib.wso_get_map_format(self._h, C.byref(v)), self._h)
+        return "rgba16f" if v.value == L.WSO_MAP_RGBA16F else "rgba32f"
 
     def GetDisplacementCount(self): return self.GetTileSize() ** 2
     def GetNormalCount(self): return self.GetTileSize() ** 2
     def GetDisplacements(self) -> np.ndarray:
-        """(N,N,4) view of the pinned host copy written by ComputeWaves (valid until the next call)."""
+        """(N,N,4) view of the pinned host copy written by ComputeWaves (valid until the next call); np.float16 with
+        RGBA16F maps."""
         return self._host_map(L.WSO_MAP_DISPLACEMENT)
     def GetNormals(self) -> np.ndarray:
         return self._host_map(L.WSO_MAP_NORMAL)
@@ -239,16 +262,22 @@ class WSTessendorf:
         L.check(self._lib.wso_compute_batch(self._h, t.size, _ptr(tl), _ptr(t), int(first_slot)), self._h)
 
     def compute_to_host(self, times, disp_out: np.ndarray, norm_out: np.ndarray, tiles=None):
-        """Streams every tile-frame's maps into host arrays (ideally PinnedBuffer.array). -> (A, min, max)"""
+        """Streams every tile-frame's maps into host arrays (ideally PinnedBuffer.array, np.float16 with RGBA16F maps).
+        -> (A, min, max)"""
         t = np.ascontiguousarray(times, np.float32)
         tl = None if tiles is None else np.ascontiguousarray(tiles, np.uint32)
         a = np.zeros(t.size, np.float32)
         mn = np.zeros(t.size, np.float32)
         mx = np.zeros(t.size, np.float32)
-        assert disp_out.dtype == np.float32 and norm_out.dtype == np.float32
+        assert disp_out.dtype == self._map_dtype and norm_out.dtype == self._map_dtype
         assert disp_out.flags.c_contiguous and norm_out.flags.c_contiguous
         need = t.size * self.GetTileSize() ** 2 * 4
         assert disp_out.size >= need and norm_out.size >= need
+        if self._map_dtype is np.float16:
+            L.check(self._lib.wso_compute_to_host_bytes(self._h, t.size, _ptr(tl), _ptr(t), _ptr(disp_out),
+                                                        _ptr(norm_out), min(disp_out.nbytes, norm_out.nbytes),
+                                                        _ptr(a), _ptr(mn), _ptr(mx)), self._h)
+            return a, mn, mx
         L.check(self._lib.wso_compute_to_host(self._h, t.size, _ptr(tl), _ptr(t), _ptr(disp_out),
                                               _ptr(norm_out), _ptr(a), _ptr(mn), _ptr(mx)), self._h)
         return a, mn, mx
@@ -265,6 +294,10 @@ class WSTessendorf:
 
     def copy_map(self, which: int, slot: int = 0) -> np.ndarray:
         n = self.GetTileSize()
+        if self._map_dtype is np.float16:
+            out = np.empty((n, n, 4), np.float16)
+            L.check(self._lib.wso_copy_map_bytes(self._h, which, slot, _ptr(out), out.nbytes), self._h)
+            return out
         out = np.empty((n, n, 4), np.float32)
         L.check(self._lib.wso_copy_map(self._h, which, slot, _ptr(out)), self._h)
         return out
@@ -280,7 +313,7 @@ class WSTessendorf:
         L.check(self._lib.wso_set_exportable(self._h, 1 if on else 0), self._h)
 
     def export_fd(self, which: int):
-        """-> (fd, bytes) of the whole [slot][N*N] RGBA32F array of one map; the caller owns the fd."""
+        """-> (fd, bytes) of the whole [slot][N*N] array of one map (RGBA32F, or RGBA16F); the caller owns the fd."""
         fd, nbytes = C.c_int(-1), C.c_size_t()
         L.check(self._lib.wso_export_fd(self._h, which, C.byref(fd), C.byref(nbytes)), self._h)
         return int(fd.value), int(nbytes.value)
