@@ -125,6 +125,13 @@ public:
     // code there) at run time - displacement.w = Jacobian of the horizontal displacement instead of 1.
     void SetComputeJacobian(bool on) { Check(wso_set_compute_jacobian(m_Ctx, on ? 1 : 0), "wso_set_compute_jacobian"); }
     void SetDamping(float damping) { Set([&](wso_params& p) { p.damping = damping; }); }
+    // Extension (not in the reference class): the surface above n world points xz[2i], xz[2i+1] (host arrays) - height,
+    // normal and undisplaced origin - sampled from the maps of the last ComputeWaves() (slot 0), with `iterations`
+    // fixed-point steps of the choppy-displacement inversion (wsocean.h, "Surface queries").  Blocking.
+    void QuerySurface(const float* xz, uint32_t n, wso_surface_sample* out, uint32_t iterations = 4) {
+        const uint32_t slot = 0;
+        Check(wso_query_surface_host(m_Ctx, 1, &slot, iterations, n, xz, out), "wso_query_surface_host");
+    }
 
     // ---- extensions: device pointers for zero-copy consumers (e.g. Vulkan external memory, row f-2)
     void* GetDisplacementsDevice() const { return DevicePtr(WSO_MAP_DISPLACEMENT); }

@@ -189,6 +189,48 @@ WSO_API int wso_compute_to_host_bytes(wso_ctx* ctx, uint32_t n, const uint32_t* 
                                       float* min_height, float* max_height);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Surface queries (an extension): height, normal and undisplaced origin of the surface at arbitrary world points
+ * (buoyancy, collision, spray, wake placement), sampled on the device from the maps of 1..4 slots (cascades: tiles of
+ * different tile_length, e.g. the tiles of a max_tiles context, each computed into its own slot), in either map format.
+ * Slot s was last written by a compute of tile t; N = tile size, L_s = tile_length t was PREPARED with, l_s = lambda in
+ * effect for that compute, A_s = that frame's amplitude (wso_read_heights), D_s / G_s = its displacement / normal map
+ * (RGBA16F decoded to fp32).
+ *   Coordinates: texel [m][n] is the field at world (x, z) = (n*L/N, m*L/N) (rows = z, columns = x), L-periodic.
+ *   Sampling S_s[F](x, z): u = x*N/L_s, v = z*N/L_s, n0 = floor(u), m0 = floor(v), fu = u - n0, fv = v - m0; bilinear
+ *       blend of texels [m0|m0+1][n0|n0+1], indices wrapped mod N (any x, z, negative or many tiles away).  x and z are
+ *       reduced mod L_s once per cascade in float64; the rest is fp32, so far-away queries are as accurate as near ones.
+ *   Inversion: choppy displacement moves points sideways.  The surface point above q = (x, z) started at p with
+ *       p + Dh(p) = q, Dh(p) = sum_s (S_s[D.x](p), S_s[D.z](p)) (D.x, D.z carry lambda).  `iterations` = I fixed-point
+ *       steps held as offsets from q:  d_0 = 0, d_{k+1} = -Dh(q + d_k), p = q + d_I.  I = 0: the point that started at q.
+ *   Record (32 bytes):
+ *       height   = sum_s A_s * S_s[D.y](p)
+ *       normal   = normalize(-sx/ex, 1, -sz/ez), sx = sum_s S_s[G.x](p), sz = sum_s S_s[G.y](p),
+ *                  ex = 1 + sum_s l_s*S_s[G.z](p), ez = 1 + sum_s l_s*S_s[G.w](p)   (one slot: the reference's vertex
+ *                  shader normal, WaterSurfaceMesh.vert:33-38)
+ *       offset   = d_I = p - q
+ *       residual = |d_I + Dh(p)|, world units: how far the answer is from q.  Where the surface folds (J < 0) the
+ *                  iteration need not converge; a large residual says so, it is not an error.
+ *       w        = S_{s0}[D.w](p) of the first slot: 1, or J if that frame had the Jacobian on.
+ * wso_query_surface: xz_dev = n (x, z) float pairs, out_dev = n records (16-byte aligned), both device pointers;
+ *   asynchronous on the context's stream, ONE kernel launch, so it follows a compute on that stream without a host sync.
+ * wso_query_surface_host: host pointers; blocking; stages through library-owned device memory grown on demand.
+ * 1 <= n_slots <= 4, iterations <= 16, n == 0 is a no-op.  WSO_ERR_INVALID_ARG (state unchanged): a slot >= max_slots, a
+ * slot that holds no computed frame (every compute entry point records one; wso_set_map_format, wso_set_exportable,
+ * wso_import_external_fd and a Prepare that changes the tile size clear them all), a NULL pointer, a misaligned out_dev,
+ * a limit exceeded.  Non-finite coordinates give NaN records (device data is not inspected).  Not on the slab path. */
+typedef struct wso_surface_sample {
+    float height;
+    float normal_x, normal_y, normal_z;
+    float offset_x, offset_z;
+    float residual;
+    float w;
+} wso_surface_sample;
+WSO_API int wso_query_surface(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, uint32_t iterations,
+                              uint32_t n, const float* xz_dev, wso_surface_sample* out_dev);
+WSO_API int wso_query_surface_host(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, uint32_t iterations,
+                                   uint32_t n, const float* xz_host, wso_surface_sample* out_host);
+
+/* ------------------------------------------------------------------------------------------------------------
  * External-memory interop (SURVEY row f-2): the maps land in memory a Vulkan device can bind, so the renderer's
  * vkCmdCopyBufferToImage reads them where K2 wrote them.  Replaces: the two 16*N*N-byte memcpy calls into the mapped
  * staging buffer and the PCIe upload behind them (WaterSurfaceMesh.cpp:701-755, vulkan/Texture2D.cpp:175-226).

@@ -27,6 +27,10 @@ WSO_MAP_NORMAL = 1
 WSO_MAP_RGBA32F = 0
 WSO_MAP_RGBA16F = 1
 
+# struct wso_surface_sample (include/wsocean.h): one 32-byte record per surface query
+SURFACE_SAMPLE_DTYPE = [("height", "<f4"), ("normal_x", "<f4"), ("normal_y", "<f4"), ("normal_z", "<f4"),
+                        ("offset_x", "<f4"), ("offset_z", "<f4"), ("residual", "<f4"), ("w", "<f4")]
+
 STATUS_NAMES = {
     0: "WSO_OK", -1: "WSO_ERR_INVALID_ARG", -2: "WSO_ERR_BAD_TILE_SIZE", -3: "WSO_ERR_NOT_PREPARED",
     -4: "WSO_ERR_CUDA", -5: "WSO_ERR_OUT_OF_MEMORY", -6: "WSO_ERR_H0_NOT_CONJUGATE",
@@ -84,6 +88,9 @@ SYMBOLS = {
     "wso_map_host_bytes": (_int, [_vp, _int, C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "wso_copy_map_bytes": (_int, [_vp, _int, _u32, _vp, C.c_size_t]),
     "wso_compute_to_host_bytes": (_int, [_vp, _u32, _vp, _vp, _vp, _vp, C.c_size_t, _vp, _vp, _vp]),
+    # surface queries (height / normal / undisplaced origin at world points, 1..4 cascades)
+    "wso_query_surface": (_int, [_vp, _u32, _vp, _u32, _u32, _vp, _vp]),
+    "wso_query_surface_host": (_int, [_vp, _u32, _vp, _u32, _u32, _vp, _vp]),
     # external-memory interop (Vulkan side of the maps)
     "wso_set_exportable": (_int, [_vp, _int]),
     "wso_export_fd": (_int, [_vp, _int, C.POINTER(_int), C.POINTER(C.c_size_t)]),

@@ -17,9 +17,10 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB_PATH = os.path.join(PKG_DIR, "libwsocean.so")
 
-SOURCES = ["wso_kernels.cu", "wso_kernels2.cu", "wso_slab_kernels.cu", "wso_prepare_kernels.cu", "wso_api.cu", "wso_slab.cu",
-           "wso_host_prepare.cpp"]
-HEADERS = ["wso_device.cuh", "wso_kernels.cuh", "wso_kernels2.cuh", "wso_simt.cuh", "wso_launch.h", "wso_host_prepare.h"]
+SOURCES = ["wso_kernels.cu", "wso_kernels2.cu", "wso_slab_kernels.cu", "wso_prepare_kernels.cu", "wso_query_kernels.cu",
+           "wso_api.cu", "wso_slab.cu", "wso_host_prepare.cpp"]
+HEADERS = ["wso_device.cuh", "wso_kernels.cuh", "wso_kernels2.cuh", "wso_simt.cuh", "wso_launch.h", "wso_host_prepare.h",
+           "wso_query.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -13,7 +13,10 @@
 #include "wso_host_prepare.h"
 #include "wso_kernels.cuh"
 #include "wso_launch.h"
+#include "wso_query.cuh"
 #include "wsocean.h"
+
+static_assert(sizeof(wso_surface_sample) == 2 * sizeof(float4), "one query record = two float4 stores");
 
 using wso::BatchItem;
 using wso::LaunchArgs;
@@ -29,6 +32,14 @@ struct Tile {
     wso_params prepared;        // parameters the resident h0 was built with
     bool is_prepared = false;
     std::vector<wso_h0_record> h0;  // host copy in the reference layout (export / checkpoint)
+};
+
+// What a map slot holds, for the surface queries: whether a compute has written it since its maps were last reset, the
+// tile_length of the tile that compute used (as prepared) and the lambda in effect.  Host-side bookkeeping only.
+struct SlotFrame {
+    bool valid = false;
+    float length = 0.0f;
+    float lambda = 0.0f;
 };
 
 enum BackingKind { kBackCudaMalloc = 0, kBackExportable = 1, kBackExternal = 2 };
@@ -76,6 +87,10 @@ struct wso_ctx {
     float4* d_norm = nullptr;
     float* d_minmax = nullptr;   // [slot][2]
     float* d_ampl = nullptr;     // [slot]
+    std::vector<SlotFrame> slot_frames;  // [slot] (wso_query_surface)
+    float* d_query_xz = nullptr;         // wso_query_surface_host staging, grown on demand: query_cap queries
+    float4* d_query_out = nullptr;
+    size_t query_cap = 0;
     // how each map array (0 = displacement, 1 = normal) is backed: cudaMalloc, an exportable virtual-memory
     // allocation, or memory imported from another API (wso_set_exportable / wso_import_external_fd)
     MapBacking map_mem[2];
@@ -186,7 +201,13 @@ char* map_slot(wso_ctx* c, int which, uint32_t slot) {
     return reinterpret_cast<char*>(map_ptr(c, which)) + map_slot_bytes(c) * slot;
 }
 
+// Every slot's maps are gone or reset: no slot holds a queryable frame until the next compute writes it.
+void forget_frames(wso_ctx* c) {
+    for (SlotFrame& f : c->slot_frames) f = SlotFrame{};
+}
+
 void free_map(wso_ctx* c, int which) {
+    forget_frames(c);
     MapBacking& b = c->map_mem[which];
     float4*& p = map_ptr(c, which);
     if (p != nullptr) {
@@ -272,6 +293,7 @@ void free_device_buffers(wso_ctx* c) {
 // displacement (0,0,0,0), normal (0,1,0,0) - in every device slot and in the pinned host mirrors of slot 0.
 // RGBA16F: the same values in binary16, normal (0, 1, 0, 0) = halves (0x0000, 0x3c00, 0x0000, 0x0000).
 int reset_map_contents(wso_ctx* c, size_t n2, int which_mask = 3) {
+    forget_frames(c);
     const size_t tb = map_texel_bytes(c);
     if (which_mask & 1) {
         WSO_CUDA(c, cudaMemsetAsync(c->d_disp, 0, tb * n2 * c->max_slots, c->stream));
@@ -518,6 +540,10 @@ int enqueue_chunk(wso_ctx* c, uint32_t n_items, const uint32_t* tiles, const flo
     if (e != cudaSuccess) return fail_cuda(c, e, "kernel launch");
     c->first_use = false;
     c->launches += (uint64_t)wso::kernels_per_launch();
+    for (uint32_t i = 0; i < n_items; ++i) {
+        const uint32_t tl = args.items[i].tile;
+        c->slot_frames[args.items[i].slot] = SlotFrame{true, c->tiles[tl].prepared.tile_length, args.td[i].lambda};
+    }
     return WSO_OK;
 }
 
@@ -613,6 +639,7 @@ int wso_create(const wso_params* p, int device, uint32_t max_tiles, uint32_t max
     c->max_tiles = max_tiles;
     c->max_slots = max_slots;
     c->tiles.resize(max_tiles);
+    c->slot_frames.resize(max_slots);
     wso_params p0 = *p;
     wso::normalise_like_setters(p0, nullptr);
     for (auto& tl : c->tiles) tl.params = p0;
@@ -662,6 +689,8 @@ int wso_destroy(wso_ctx* c) {
     if (c->aux_stream) cudaStreamSynchronize(c->aux_stream);
     wso::destroy_frame_graph(c->frame_graph);
     free_device_buffers(c);
+    cudaFree(c->d_query_xz);
+    cudaFree(c->d_query_out);
     for (int i = 0; i < 2; ++i)
         if (c->ext_sem[i]) cudaDestroyExternalSemaphore(c->ext_sem[i]);
     if (c->ev_async) cudaEventDestroy(c->ev_async);
@@ -1154,6 +1183,84 @@ int wso_set_map_format(wso_ctx* c, int format) {
 int wso_get_map_format(const wso_ctx* c, int* format) {
     if (!c || !format) return WSO_ERR_INVALID_ARG;
     *format = c->map_format;
+    return WSO_OK;
+}
+
+}  // extern "C"
+
+namespace {
+
+// Everything wso_query_surface checks before it touches the device; fills the cascade constants of a launch.
+int check_query(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, uint32_t iterations, wso::QueryArgs* a) {
+    if (!c) return WSO_ERR_INVALID_ARG;
+    if (!slots) return fail(c, WSO_ERR_INVALID_ARG, "slots is NULL");
+    if (n_slots < 1 || n_slots > (uint32_t)wso::kMaxQueryCascades)
+        return fail(c, WSO_ERR_INVALID_ARG, "n_slots must be 1..4");
+    if (iterations > (uint32_t)wso::kMaxQueryIterations) return fail(c, WSO_ERR_INVALID_ARG, "iterations must be <= 16");
+    *a = wso::QueryArgs{};
+    for (uint32_t i = 0; i < n_slots; ++i) {
+        const uint32_t s = slots[i];
+        if (s >= c->max_slots) return fail(c, WSO_ERR_INVALID_ARG, "slot out of range");
+        const SlotFrame& f = c->slot_frames[s];
+        if (!f.valid || c->n == 0)
+            return fail(c, WSO_ERR_INVALID_ARG, "slot " + std::to_string(s) + " holds no computed frame");
+        a->c[i] = wso::make_query_cascade(map_slot(c, 0, s), map_slot(c, 1, s), c->d_ampl + s, c->n, f.length, f.lambda);
+    }
+    a->mask = c->n - 1;
+    a->logn = c->logn;
+    a->iterations = (int)iterations;
+    return WSO_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int wso_query_surface(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, uint32_t iterations, uint32_t n,
+                      const float* xz_dev, wso_surface_sample* out_dev) {
+    wso::QueryArgs a;
+    int rc = check_query(c, n_slots, slots, iterations, &a);
+    if (rc != WSO_OK) return rc;
+    if (n == 0) return WSO_OK;
+    if (!xz_dev || !out_dev) return fail(c, WSO_ERR_INVALID_ARG, "xz or out is NULL");
+    if (reinterpret_cast<uintptr_t>(out_dev) % 16 != 0) return fail(c, WSO_ERR_INVALID_ARG, "out is not 16-byte aligned");
+    a.xz = xz_dev;
+    a.out = reinterpret_cast<float4*>(out_dev);
+    a.n = n;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    WSO_CUDA(c, wso::launch_query_surface(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    return WSO_OK;
+}
+
+int wso_query_surface_host(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, uint32_t iterations, uint32_t n,
+                           const float* xz_host, wso_surface_sample* out_host) {
+    wso::QueryArgs a;
+    int rc = check_query(c, n_slots, slots, iterations, &a);
+    if (rc != WSO_OK) return rc;
+    if (n == 0) return WSO_OK;
+    if (!xz_host || !out_host) return fail(c, WSO_ERR_INVALID_ARG, "xz or out is NULL");
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    if (n > c->query_cap) {
+        WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+        cudaFree(c->d_query_xz);
+        cudaFree(c->d_query_out);
+        c->d_query_xz = nullptr;
+        c->d_query_out = nullptr;
+        c->query_cap = 0;
+        WSO_CUDA(c, cudaMalloc(&c->d_query_xz, sizeof(float) * 2 * (size_t)n));
+        WSO_CUDA(c, cudaMalloc(&c->d_query_out, sizeof(wso_surface_sample) * (size_t)n));
+        c->query_cap = n;
+    }
+    WSO_CUDA(c, cudaMemcpyAsync(c->d_query_xz, xz_host, sizeof(float) * 2 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+    a.xz = c->d_query_xz;
+    a.out = c->d_query_out;
+    a.n = n;
+    WSO_CUDA(c, wso::launch_query_surface(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_query_out, sizeof(wso_surface_sample) * (size_t)n, cudaMemcpyDeviceToHost,
+                                c->stream));
+    WSO_CUDA(c, cudaStreamSynchronize(c->stream));
     return WSO_OK;
 }
 

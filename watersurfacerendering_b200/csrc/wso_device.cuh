@@ -130,6 +130,33 @@ WSO_HD uint16_t f32_to_f16_rn(float x) {
     if (rem > half || (rem == half && (r & 1u))) ++r;  // may carry into the smallest normal, 0x0400: still right
     return (uint16_t)(sign | r);
 }
+
+// Portable binary16 bits -> float (exact: every binary16 value is a float), for the host build of the query body
+// (wso_query.cuh) reading RGBA16F maps.
+WSO_HD float f16_to_f32(uint16_t h) {
+    const uint32_t sign = (uint32_t)(h & 0x8000u) << 16;
+    const uint32_t e = (h >> 10) & 0x1fu, m = h & 0x3ffu;
+    uint32_t u;
+    if (e == 0x1fu) {
+        u = sign | 0x7f800000u | (m << 13);  // inf, NaN (payload kept)
+    } else if (e != 0u) {
+        u = sign | ((e + 112u) << 23) | (m << 13);  // normal: rebias 15 -> 127
+    } else if (m == 0u) {
+        u = sign;  // signed zero
+    } else {
+        // subnormal m * 2^-24: shift the leading one up to bit 10, lowering the exponent of 2^-14 once per step
+        uint32_t ex = 113u;
+        uint32_t mm = m;
+        while ((mm & 0x400u) == 0u) {
+            mm <<= 1;
+            --ex;
+        }
+        u = sign | (ex << 23) | ((mm & 0x3ffu) << 13);
+    }
+    float f;
+    memcpy(&f, &u, 4);
+    return f;
+}
 #endif
 
 // binary16 bits of (lo, hi) in one 32-bit word, lo in bits 0..15

@@ -88,4 +88,9 @@ cudaError_t launch_prepare(const PrepareArgs& a, int n_pairs, cudaStream_t strea
 cudaError_t launch_export_records(const float4* h0, float* out20, int n, float omega0, bool table, cudaStream_t stream);
 uint64_t counter_seed_mix(uint64_t seed);
 
+// Surface queries (wso_query_kernels.cu, body in wso_query.cuh): one launch, one thread per query over args.c[0..n_slots)
+// (1..4 cascades); half: the maps hold RGBA16F texels.  args.n > 0.
+struct QueryArgs;
+cudaError_t launch_query_surface(const QueryArgs& args, int n_slots, bool half, cudaStream_t stream);
+
 }  // namespace wso

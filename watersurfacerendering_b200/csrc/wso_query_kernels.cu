@@ -1,0 +1,45 @@
+// wso_query_kernels.cu — the surface-query kernel (wso_query_surface): one thread per query, the per-query body of
+// wso_query.cuh, the cascade constants in a __grid_constant__ parameter block.  Texel loads go through the read-only
+// non-coherent path (the maps of every cascade together are a few MB at 512^2 / 1024^2 and stay L2-resident across
+// queries); each record leaves as two 16-byte stores.
+#include <cuda_runtime.h>
+#include <stdint.h>
+
+#include "wso_query.cuh"
+
+namespace wso {
+
+namespace {
+
+template <class Texel, int NS>
+__global__ void __launch_bounds__(256) wso_query_kernel(const __grid_constant__ QueryArgs a) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    const float qx = __ldg(a.xz + 2 * (size_t)i), qz = __ldg(a.xz + 2 * (size_t)i + 1);
+    float4 o[2];
+    query_point<Texel, NS>(a, qx, qz, o);
+    a.out[2 * (size_t)i] = o[0];
+    a.out[2 * (size_t)i + 1] = o[1];
+}
+
+template <class Texel>
+cudaError_t launch_texel(const QueryArgs& a, int n_slots, cudaStream_t stream) {
+    const unsigned threads = 256;
+    const unsigned blocks = (unsigned)((a.n + threads - 1) / threads);
+    switch (n_slots) {
+        case 1: wso_query_kernel<Texel, 1><<<blocks, threads, 0, stream>>>(a); break;
+        case 2: wso_query_kernel<Texel, 2><<<blocks, threads, 0, stream>>>(a); break;
+        case 3: wso_query_kernel<Texel, 3><<<blocks, threads, 0, stream>>>(a); break;
+        case 4: wso_query_kernel<Texel, 4><<<blocks, threads, 0, stream>>>(a); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_query_surface(const QueryArgs& a, int n_slots, bool half, cudaStream_t stream) {
+    return half ? launch_texel<Half4>(a, n_slots, stream) : launch_texel<float4>(a, n_slots, stream);
+}
+
+}  // namespace wso

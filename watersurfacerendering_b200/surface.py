@@ -18,6 +18,8 @@ from . import _lib as L
 H0_DTYPE = np.dtype(
     [("re", "<f4"), ("im", "<f4"), ("re_c", "<f4"), ("im_c", "<f4"), ("omega", "<f4")]
 )
+# wso_surface_sample: height, normal (x, y, z), offset (x, z) = undisplaced origin - query, residual, w
+SURFACE_SAMPLE_DTYPE = np.dtype(L.SURFACE_SAMPLE_DTYPE)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -306,6 +308,31 @@ class WSTessendorf:
         p, cnt = C.c_void_p(), C.c_size_t()
         L.check(self._lib.wso_map_device(self._h, which, slot, C.byref(p), C.byref(cnt)), self._h)
         return int(p.value)
+
+    # ---- surface queries (extension: the surface at arbitrary world points, sampled on the device)
+    @staticmethod
+    def _slots(slots):
+        sl = np.ascontiguousarray(np.atleast_1d(np.asarray(slots)), np.uint32)
+        return sl, int(sl.size)
+
+    def query_surface(self, xz, slots=(0,), iterations: int = 4) -> np.ndarray:
+        """Height, normal and undisplaced origin of the surface above the world points xz ((n, 2) or (2,) array of
+        (x, z)), summed over the cascades `slots` (1..4 slots holding computed frames), with `iterations` fixed-point steps
+        of the choppy-displacement inversion.  Blocking (wso_query_surface_host).  -> structured array of n records
+        (SURFACE_SAMPLE_DTYPE: height, normal_x/y/z, offset_x/z, residual, w)."""
+        q = np.ascontiguousarray(xz, np.float32).reshape(-1, 2)
+        out = np.zeros(q.shape[0], SURFACE_SAMPLE_DTYPE)
+        sl, ns = self._slots(slots)
+        L.check(self._lib.wso_query_surface_host(self._h, ns, _ptr(sl), int(iterations), q.shape[0], _ptr(q),
+                                                 _ptr(out)), self._h)
+        return out
+
+    def query_surface_device(self, xz_ptr: int, out_ptr: int, n: int, slots=(0,), iterations: int = 4):
+        """The same on device memory (e.g. tensor.data_ptr()): xz_ptr = n (x, z) float pairs, out_ptr = n 32-byte records
+        (16-byte aligned).  Asynchronous on the context's stream (wso_query_surface)."""
+        sl, ns = self._slots(slots)
+        L.check(self._lib.wso_query_surface(self._h, ns, _ptr(sl), int(iterations), int(n), C.c_void_p(xz_ptr or 0),
+                                            C.c_void_p(out_ptr or 0)), self._h)
 
     # ---- external-memory interop (SURVEY row f-2; replaces the staging memcpy of WaterSurfaceMesh.cpp:701-755)
     def set_exportable(self, on: bool = True):
