@@ -132,6 +132,12 @@ public:
         const uint32_t slot = 0;
         Check(wso_query_surface_host(m_Ctx, 1, &slot, iterations, n, xz, out), "wso_query_surface_host");
     }
+    // Extension: the first point at or under the surface of slot 0 along n rays, rays[8i..8i+7] = (ox, oy, oz, tmax,
+    // dx, dy, dz, unused) (host arrays), marched and refined as `p` says (wsocean.h, "Ray casts").  Blocking.
+    void RaycastSurface(const float* rays, uint32_t n, wso_ray_hit* out, const wso_ray_params& p) {
+        const uint32_t slot = 0;
+        Check(wso_raycast_surface_host(m_Ctx, 1, &slot, &p, n, rays, out), "wso_raycast_surface_host");
+    }
 
     // ---- extensions: device pointers for zero-copy consumers (e.g. Vulkan external memory, row f-2)
     void* GetDisplacementsDevice() const { return DevicePtr(WSO_MAP_DISPLACEMENT); }

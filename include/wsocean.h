@@ -231,6 +231,60 @@ WSO_API int wso_query_surface_host(wso_ctx* ctx, uint32_t n_slots, const uint32_
                                    uint32_t n, const float* xz_host, wso_surface_sample* out_host);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Ray casts (an extension): the first point of a segment at or under the displaced surface (projectiles, line of
+ * sight, picking, camera under water), marched on the device over the same 1..4 slots as the surface queries.
+ * H(q) below is the height of a surface query (same slots, same iterations I) evaluated at slot-local positions q_s.
+ * All fp32 operations are round-to-nearest and happen in this order ("fl" = one rounding):
+ *   Ray: o = (ox, oy, oz), range tmax, direction d.  m = max(|dx|, |dy|, |dz|); v = fl(d / m) per component;
+ *       len = fl(sqrt(fl(fl(vx*vx + vy*vy) + vz*vz))); d^ = fl(v / len) per component.
+ *   INVALID: o or d has a non-finite component, d = 0, or tmax is NaN or negative (+inf is allowed).  distance, x, z
+ *       and the sample are NaN.  Rays are checked one by one on the device: bad data is never a call error.
+ *   Slab: Hb = fl(fl(sum_s |A_s|) * (1 + 2^-10)) > |every height a query or the march can return| (proof in
+ *       csrc/wso_query.cuh).  oy < -Hb: ORIGIN_BELOW.  Otherwise, d^y != 0: t1 = fl(fl(Hb - oy) / d^y),
+ *       t2 = fl(fl(-Hb - oy) / d^y), entry = min, exit = max; d^y = 0: entry = -inf, exit = +inf if oy <= Hb else -inf.
+ *       s0 = max(0, entry), s_end = min(tmax, exit).  s0 > s_end: MISS without any sample.
+ *   March positions: per cascade p_s = (reduce_mod(ox, L_s), reduce_mod(oz, L_s)) (float64 mod L_s, rounded once, as
+ *       the queries do); at parameter t: q_s = (fl(p_s.x + fl(t*d^x)), fl(p_s.z + fl(t*d^z))), y = fl(oy + fl(t*d^y)).
+ *       The point is at or under the surface, f(t) <= 0, when y <= H(q).  Accuracy depends on the distance marched,
+ *       not on |o|.
+ *   March: t_k = fl(s0 + fl(k*step)) for k = 0, 1, ... while t_k < s_end, then t = s_end; at most max_steps samples.
+ *       The first sample with f <= 0 ends the march: at k = 0 with s0 = 0 it is ORIGIN_BELOW; otherwise a HIT
+ *       bracketed by [a, b] = [previous sample, this sample] (at k = 0 with s0 > 0: [s0, s0]).  The sample at s_end
+ *       with f > 0: MISS.  max_steps samples taken before s_end: UNRESOLVED.
+ *   Refine (HIT): `refine` times m = fl(a + fl(0.5 * fl(b - a))); f(m) > 0 ? a = m : b = m.  distance = b: a point
+ *       at or under the surface at most step * 2^-refine past the first sign change the march saw.
+ *   Record (48 bytes): HIT / ORIGIN_BELOW (distance b = 0): x = fl(ox + fl(b*d^x)), z = fl(oz + fl(b*d^z)) and
+ *       `surface` = bit for bit the wso_surface_sample wso_query_surface returns at (x, z) with the same slots and
+ *       iterations (surface.height is the hit's y).  MISS: distance +inf.  UNRESOLVED: distance = the parameter of the
+ *       last sample; continue with origin o + distance*d^ and range tmax - distance.  Both: x, z, surface NaN.
+ * A march step costs one H evaluation: 4 * n_slots * (I + 1) displacement texels; the normal maps are read only for
+ * the record.  Choose step at most the finest texel spacing L_s/N: a ray can pass through a wave crest thinner than
+ * step between two samples without seeing it (tunnelling).
+ * wso_raycast_surface: rays_dev = n x 8 floats (ox, oy, oz, tmax, dx, dy, dz, unused), out_dev = n records, device
+ *   pointers, both 16-byte aligned; asynchronous on the context's stream, ONE kernel launch.
+ * wso_raycast_surface_host: host pointers; blocking; stages through library-owned device memory grown on demand.
+ * WSO_ERR_INVALID_ARG (state unchanged): everything wso_query_surface rejects (slots, n_slots, iterations > 16), a NULL
+ * p, step not finite and > 0, max_steps outside 1..4096, refine > 24, a NULL or misaligned pointer.  n == 0 is a no-op.
+ * Not on the slab path. */
+typedef struct wso_ray_params {
+    float step;           /* march spacing along the ray, world units, finite and > 0 */
+    uint32_t max_steps;   /* march samples per ray, 1..4096 */
+    uint32_t refine;      /* bisection steps after a bracket, 0..24 */
+    uint32_t iterations;  /* inversion steps of every H evaluation, 0..16 (as wso_query_surface) */
+} wso_ray_params;
+enum { WSO_RAY_MISS = 0, WSO_RAY_HIT = 1, WSO_RAY_ORIGIN_BELOW = 2, WSO_RAY_UNRESOLVED = 3, WSO_RAY_INVALID = 4 };
+typedef struct wso_ray_hit {
+    float distance;               /* along d^: b (hit), 0 (origin below), +inf (miss), last sample (unresolved), NaN */
+    float x, z;                   /* world position of the hit */
+    uint32_t status;              /* WSO_RAY_* */
+    wso_surface_sample surface;   /* wso_query_surface at (x, z) */
+} wso_ray_hit;
+WSO_API int wso_raycast_surface(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, const wso_ray_params* p,
+                                uint32_t n, const float* rays_dev, wso_ray_hit* out_dev);
+WSO_API int wso_raycast_surface_host(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, const wso_ray_params* p,
+                                     uint32_t n, const float* rays_host, wso_ray_hit* out_host);
+
+/* ------------------------------------------------------------------------------------------------------------
  * External-memory interop (SURVEY row f-2): the maps land in memory a Vulkan device can bind, so the renderer's
  * vkCmdCopyBufferToImage reads them where K2 wrote them.  Replaces: the two 16*N*N-byte memcpy calls into the mapped
  * staging buffer and the PCIe upload behind them (WaterSurfaceMesh.cpp:701-755, vulkan/Texture2D.cpp:175-226).

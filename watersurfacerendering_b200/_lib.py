@@ -31,6 +31,16 @@ WSO_MAP_RGBA16F = 1
 SURFACE_SAMPLE_DTYPE = [("height", "<f4"), ("normal_x", "<f4"), ("normal_y", "<f4"), ("normal_z", "<f4"),
                         ("offset_x", "<f4"), ("offset_z", "<f4"), ("residual", "<f4"), ("w", "<f4")]
 
+# ray casts (wso_raycast_surface): status of a wso_ray_hit
+WSO_RAY_MISS = 0
+WSO_RAY_HIT = 1
+WSO_RAY_ORIGIN_BELOW = 2
+WSO_RAY_UNRESOLVED = 3
+WSO_RAY_INVALID = 4
+
+# struct wso_ray_hit (include/wsocean.h): one 48-byte record per ray, the hit's wso_surface_sample flattened into it
+RAY_HIT_DTYPE = [("distance", "<f4"), ("x", "<f4"), ("z", "<f4"), ("status", "<u4")] + SURFACE_SAMPLE_DTYPE
+
 STATUS_NAMES = {
     0: "WSO_OK", -1: "WSO_ERR_INVALID_ARG", -2: "WSO_ERR_BAD_TILE_SIZE", -3: "WSO_ERR_NOT_PREPARED",
     -4: "WSO_ERR_CUDA", -5: "WSO_ERR_OUT_OF_MEMORY", -6: "WSO_ERR_H0_NOT_CONJUGATE",
@@ -49,6 +59,16 @@ class WsoParams(C.Structure):
         ("phillips_const", C.c_float),
         ("damping", C.c_float),
         ("lambda_", C.c_float),
+    ]
+
+
+class WsoRayParams(C.Structure):
+    """struct wso_ray_params (include/wsocean.h)."""
+    _fields_ = [
+        ("step", C.c_float),
+        ("max_steps", C.c_uint32),
+        ("refine", C.c_uint32),
+        ("iterations", C.c_uint32),
     ]
 
 
@@ -91,6 +111,9 @@ SYMBOLS = {
     # surface queries (height / normal / undisplaced origin at world points, 1..4 cascades)
     "wso_query_surface": (_int, [_vp, _u32, _vp, _u32, _u32, _vp, _vp]),
     "wso_query_surface_host": (_int, [_vp, _u32, _vp, _u32, _u32, _vp, _vp]),
+    # ray casts (first hit of a segment with the displaced surface, 1..4 cascades)
+    "wso_raycast_surface": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
+    "wso_raycast_surface_host": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
     # external-memory interop (Vulkan side of the maps)
     "wso_set_exportable": (_int, [_vp, _int]),
     "wso_export_fd": (_int, [_vp, _int, C.POINTER(_int), C.POINTER(C.c_size_t)]),

@@ -1,4 +1,6 @@
 // wso_api.cu — the C ABI (include/wsocean.h): context, buffers, Prepare(), batching, host copies.
+#include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -17,6 +19,9 @@
 #include "wsocean.h"
 
 static_assert(sizeof(wso_surface_sample) == 2 * sizeof(float4), "one query record = two float4 stores");
+static_assert(sizeof(wso_ray_hit) == 48, "one ray record = three float4 stores");
+static_assert(WSO_RAY_INVALID == wso::kRayInvalid && WSO_RAY_UNRESOLVED == wso::kRayUnresolved && WSO_RAY_HIT == wso::kRayHit,
+              "ray status codes of the C ABI and the kernel body");
 
 using wso::BatchItem;
 using wso::LaunchArgs;
@@ -88,9 +93,9 @@ struct wso_ctx {
     float* d_minmax = nullptr;   // [slot][2]
     float* d_ampl = nullptr;     // [slot]
     std::vector<SlotFrame> slot_frames;  // [slot] (wso_query_surface)
-    float* d_query_xz = nullptr;         // wso_query_surface_host staging, grown on demand: query_cap queries
-    float4* d_query_out = nullptr;
-    size_t query_cap = 0;
+    void* d_stage_in = nullptr;          // staging of the blocking surface queries and ray casts, grown on demand
+    void* d_stage_out = nullptr;
+    size_t stage_in_bytes = 0, stage_out_bytes = 0;
     // how each map array (0 = displacement, 1 = normal) is backed: cudaMalloc, an exportable virtual-memory
     // allocation, or memory imported from another API (wso_set_exportable / wso_import_external_fd)
     MapBacking map_mem[2];
@@ -689,8 +694,8 @@ int wso_destroy(wso_ctx* c) {
     if (c->aux_stream) cudaStreamSynchronize(c->aux_stream);
     wso::destroy_frame_graph(c->frame_graph);
     free_device_buffers(c);
-    cudaFree(c->d_query_xz);
-    cudaFree(c->d_query_out);
+    cudaFree(c->d_stage_in);
+    cudaFree(c->d_stage_out);
     for (int i = 0; i < 2; ++i)
         if (c->ext_sem[i]) cudaDestroyExternalSemaphore(c->ext_sem[i]);
     if (c->ev_async) cudaEventDestroy(c->ev_async);
@@ -1212,6 +1217,40 @@ int check_query(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, uint32_t it
     return WSO_OK;
 }
 
+// wso_raycast_surface's checks: those of the queries plus the march parameters.
+int check_raycast(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_ray_params* p, wso::RayArgs* a) {
+    if (!c) return WSO_ERR_INVALID_ARG;
+    if (!p) return fail(c, WSO_ERR_INVALID_ARG, "ray params are NULL");
+    const int rc = check_query(c, n_slots, slots, p->iterations, &a->q);
+    if (rc != WSO_OK) return rc;
+    if (!(p->step > 0.0f && p->step <= FLT_MAX)) return fail(c, WSO_ERR_INVALID_ARG, "step must be finite and > 0");
+    if (p->max_steps < 1 || p->max_steps > wso::kMaxRaySteps)
+        return fail(c, WSO_ERR_INVALID_ARG, "max_steps must be 1..4096");
+    if (p->refine > wso::kMaxRayRefine) return fail(c, WSO_ERR_INVALID_ARG, "refine must be <= 24");
+    a->step = p->step;
+    a->max_steps = p->max_steps;
+    a->refine = p->refine;
+    return WSO_OK;
+}
+
+// The device staging of the blocking query / ray-cast forms: at least in_bytes and out_bytes, grown on demand.
+int grow_staging(wso_ctx* c, size_t in_bytes, size_t out_bytes) {
+    if (in_bytes <= c->stage_in_bytes && out_bytes <= c->stage_out_bytes) return WSO_OK;
+    in_bytes = std::max(in_bytes, c->stage_in_bytes);
+    out_bytes = std::max(out_bytes, c->stage_out_bytes);
+    WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+    cudaFree(c->d_stage_in);
+    cudaFree(c->d_stage_out);
+    c->d_stage_in = nullptr;
+    c->d_stage_out = nullptr;
+    c->stage_in_bytes = c->stage_out_bytes = 0;
+    WSO_CUDA(c, cudaMalloc(&c->d_stage_in, in_bytes));
+    WSO_CUDA(c, cudaMalloc(&c->d_stage_out, out_bytes));
+    c->stage_in_bytes = in_bytes;
+    c->stage_out_bytes = out_bytes;
+    return WSO_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1241,24 +1280,55 @@ int wso_query_surface_host(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, 
     if (n == 0) return WSO_OK;
     if (!xz_host || !out_host) return fail(c, WSO_ERR_INVALID_ARG, "xz or out is NULL");
     WSO_CUDA(c, cudaSetDevice(c->device));
-    if (n > c->query_cap) {
-        WSO_CUDA(c, cudaStreamSynchronize(c->stream));
-        cudaFree(c->d_query_xz);
-        cudaFree(c->d_query_out);
-        c->d_query_xz = nullptr;
-        c->d_query_out = nullptr;
-        c->query_cap = 0;
-        WSO_CUDA(c, cudaMalloc(&c->d_query_xz, sizeof(float) * 2 * (size_t)n));
-        WSO_CUDA(c, cudaMalloc(&c->d_query_out, sizeof(wso_surface_sample) * (size_t)n));
-        c->query_cap = n;
-    }
-    WSO_CUDA(c, cudaMemcpyAsync(c->d_query_xz, xz_host, sizeof(float) * 2 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
-    a.xz = c->d_query_xz;
-    a.out = c->d_query_out;
+    rc = grow_staging(c, sizeof(float) * 2 * (size_t)n, sizeof(wso_surface_sample) * (size_t)n);
+    if (rc != WSO_OK) return rc;
+    WSO_CUDA(c, cudaMemcpyAsync(c->d_stage_in, xz_host, sizeof(float) * 2 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+    a.xz = static_cast<const float*>(c->d_stage_in);
+    a.out = static_cast<float4*>(c->d_stage_out);
     a.n = n;
     WSO_CUDA(c, wso::launch_query_surface(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
     c->launches += 1;
-    WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_query_out, sizeof(wso_surface_sample) * (size_t)n, cudaMemcpyDeviceToHost,
+    WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_stage_out, sizeof(wso_surface_sample) * (size_t)n, cudaMemcpyDeviceToHost,
+                                c->stream));
+    WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+    return WSO_OK;
+}
+
+int wso_raycast_surface(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_ray_params* p, uint32_t n,
+                        const float* rays_dev, wso_ray_hit* out_dev) {
+    wso::RayArgs a;
+    int rc = check_raycast(c, n_slots, slots, p, &a);
+    if (rc != WSO_OK) return rc;
+    if (n == 0) return WSO_OK;
+    if (!rays_dev || !out_dev) return fail(c, WSO_ERR_INVALID_ARG, "rays or out is NULL");
+    if (reinterpret_cast<uintptr_t>(rays_dev) % 16 != 0 || reinterpret_cast<uintptr_t>(out_dev) % 16 != 0)
+        return fail(c, WSO_ERR_INVALID_ARG, "rays or out is not 16-byte aligned");
+    a.rays = reinterpret_cast<const float4*>(rays_dev);
+    a.out = reinterpret_cast<float4*>(out_dev);
+    a.n = n;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    WSO_CUDA(c, wso::launch_raycast_surface(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    return WSO_OK;
+}
+
+int wso_raycast_surface_host(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_ray_params* p, uint32_t n,
+                             const float* rays_host, wso_ray_hit* out_host) {
+    wso::RayArgs a;
+    int rc = check_raycast(c, n_slots, slots, p, &a);
+    if (rc != WSO_OK) return rc;
+    if (n == 0) return WSO_OK;
+    if (!rays_host || !out_host) return fail(c, WSO_ERR_INVALID_ARG, "rays or out is NULL");
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    rc = grow_staging(c, sizeof(float) * 8 * (size_t)n, sizeof(wso_ray_hit) * (size_t)n);
+    if (rc != WSO_OK) return rc;
+    WSO_CUDA(c, cudaMemcpyAsync(c->d_stage_in, rays_host, sizeof(float) * 8 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+    a.rays = static_cast<const float4*>(c->d_stage_in);
+    a.out = static_cast<float4*>(c->d_stage_out);
+    a.n = n;
+    WSO_CUDA(c, wso::launch_raycast_surface(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_stage_out, sizeof(wso_ray_hit) * (size_t)n, cudaMemcpyDeviceToHost,
                                 c->stream));
     WSO_CUDA(c, cudaStreamSynchronize(c->stream));
     return WSO_OK;

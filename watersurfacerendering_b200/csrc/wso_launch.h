@@ -92,5 +92,8 @@ uint64_t counter_seed_mix(uint64_t seed);
 // (1..4 cascades); half: the maps hold RGBA16F texels.  args.n > 0.
 struct QueryArgs;
 cudaError_t launch_query_surface(const QueryArgs& args, int n_slots, bool half, cudaStream_t stream);
+// Ray casts (same files): one launch, one thread per ray over args.q.c[0..n_slots).  args.n > 0.
+struct RayArgs;
+cudaError_t launch_raycast_surface(const RayArgs& args, int n_slots, bool half, cudaStream_t stream);
 
 }  // namespace wso

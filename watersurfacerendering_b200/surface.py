@@ -20,6 +20,8 @@ H0_DTYPE = np.dtype(
 )
 # wso_surface_sample: height, normal (x, y, z), offset (x, z) = undisplaced origin - query, residual, w
 SURFACE_SAMPLE_DTYPE = np.dtype(L.SURFACE_SAMPLE_DTYPE)
+# wso_ray_hit: distance, hit x / z, status (WSO_RAY_*), then the wso_surface_sample at (x, z)
+RAY_HIT_DTYPE = np.dtype(L.RAY_HIT_DTYPE)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -333,6 +335,42 @@ class WSTessendorf:
         sl, ns = self._slots(slots)
         L.check(self._lib.wso_query_surface(self._h, ns, _ptr(sl), int(iterations), int(n), C.c_void_p(xz_ptr or 0),
                                             C.c_void_p(out_ptr or 0)), self._h)
+
+    # ---- ray casts (extension: first hit of a segment with the displaced surface, marched on the device)
+    @staticmethod
+    def _ray_params(step, max_steps, refine, iterations):
+        return L.WsoRayParams(float(step), int(max_steps), int(refine), int(iterations))
+
+    def raycast_surface(self, origins, directions, tmax=np.inf, slots=(0,), *, step: float, max_steps: int = 1024,
+                        refine: int = 16, iterations: int = 4) -> np.ndarray:
+        """First point at or under the surface of each ray o + t*d/|d|, 0 <= t <= tmax: origins / directions = (n, 3)
+        or (3,) arrays of (x, y, z) (broadcast against each other), tmax a scalar or n ranges.  Marched every `step` world
+        units (at most the finest texel spacing L/N; at most `max_steps` samples), the bracket refined by `refine`
+        bisection steps, every height with `iterations` inversion steps over the cascades `slots`.  Blocking
+        (wso_raycast_surface_host).  -> structured array of n records (RAY_HIT_DTYPE: distance, x, z, status =
+        WSO_RAY_*, then the surface query at (x, z))."""
+        o, d = np.broadcast_arrays(np.atleast_2d(np.asarray(origins, np.float32)),
+                                   np.atleast_2d(np.asarray(directions, np.float32)))
+        rays = np.zeros((o.shape[0], 8), np.float32)
+        rays[:, 0:3] = o
+        rays[:, 3] = np.broadcast_to(np.asarray(tmax, np.float32), (o.shape[0],))
+        rays[:, 4:7] = d
+        out = np.zeros(rays.shape[0], RAY_HIT_DTYPE)
+        sl, ns = self._slots(slots)
+        p = self._ray_params(step, max_steps, refine, iterations)
+        L.check(self._lib.wso_raycast_surface_host(self._h, ns, _ptr(sl), C.byref(p), rays.shape[0], _ptr(rays),
+                                                   _ptr(out)), self._h)
+        return out
+
+    def raycast_surface_device(self, rays_ptr: int, out_ptr: int, n: int, slots=(0,), *, step: float,
+                               max_steps: int = 1024, refine: int = 16, iterations: int = 4):
+        """The same on device memory (e.g. tensor.data_ptr()): rays_ptr = n x 8 floats (ox, oy, oz, tmax, dx, dy, dz,
+        unused), out_ptr = n 48-byte records, both 16-byte aligned.  Asynchronous on the context's stream
+        (wso_raycast_surface)."""
+        sl, ns = self._slots(slots)
+        p = self._ray_params(step, max_steps, refine, iterations)
+        L.check(self._lib.wso_raycast_surface(self._h, ns, _ptr(sl), C.byref(p), int(n), C.c_void_p(rays_ptr or 0),
+                                              C.c_void_p(out_ptr or 0)), self._h)
 
     # ---- external-memory interop (SURVEY row f-2; replaces the staging memcpy of WaterSurfaceMesh.cpp:701-755)
     def set_exportable(self, on: bool = True):
