@@ -16,7 +16,7 @@ def lib():
     global _lib
     if _lib is None:
         deps = [os.path.join(HERE, "emu.cpp"), os.path.join(CSRC, "wso_kernels.cuh"),
-                os.path.join(CSRC, "wso_device.cuh")]
+                os.path.join(CSRC, "wso_device.cuh"), os.path.join(CSRC, "wso_tilings.h")]
         if not os.path.exists(LIB) or any(os.path.getmtime(d) > os.path.getmtime(LIB) for d in deps):
             cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
             subprocess.check_call([cxx, "-std=c++17", "-O2", "-w", "-ffp-contract=off", "-fPIC", "-shared",
@@ -31,6 +31,10 @@ def lib():
         L.wso_emu_compute_slab.restype = C.c_int
         L.wso_emu_slab_rank_phase.argtypes = [C.c_int] * 5 + [vp, vp, vp, C.c_float, C.c_float, C.c_float] + [vp] * 6
         L.wso_emu_slab_rank_phase.restype = C.c_int
+        L.wso_emu_compute_shipped.argtypes = [C.c_int] * 4 + [vp] * 11
+        L.wso_emu_compute_shipped.restype = C.c_int
+        L.wso_emu_tilings.argtypes = [vp]
+        L.wso_emu_tilings.restype = C.c_int
         _lib = L
     return _lib
 
@@ -64,6 +68,54 @@ def compute(n, tile_length, lam, h0_re, h0_im, omega, t, variant=0, want_w=False
         # paired W layout (WLayout<LOGN>::paired in wso_kernels.cuh): element 2*j + half -> canonical half*N/2 + j
         w = np.concatenate([w[:, :, 0::2], w[:, :, 1::2]], axis=2)
     return a[0], disp, norm, mm[0], mm[1], w
+
+
+# kinds of compute_shipped(): the tilings of wso_tilings.h as launch_all() in wso_kernels.cu runs them
+KIND_LAT, KIND_BULK, KIND_PERSIST, KIND_JACOBIAN = 0, 1, 2, 3
+
+
+def shipped_tilings():
+    """[(logn, kind, CP, NF, RI, RH, persist)] - every tiling launch_all() can pick (kind 0 = Lat, 1 = Bulk; persist:
+    bit 0 / bit 2 = Bulk's K1 / K2 have a persistent form), read from the header the library is built from."""
+    out = np.zeros((64, 7), np.int32)
+    n = lib().wso_emu_tilings(out.ctypes.data_as(C.c_void_p))
+    return [tuple(int(v) for v in r) for r in out[:n]]
+
+
+def compute_shipped(n, kind, items, half=False, want_w=False):
+    """One emulated launch of len(items) tile-frames through a shipped tiling.  items: dicts with keys re, im, omega
+    ((N,N) reference layout [m][n]), tile_length, lam, t and optional anim_period (None: no sincos table).
+    Returns (A[k], disp[k,N,N,4], norm[k,N,N,4], min[k], max[k], W) - maps as float32 (RGBA16F maps widened)."""
+    logn = int(np.log2(n))
+    k = len(items)
+    amp_t = np.ascontiguousarray(np.stack([np.stack([it["re"].T, it["im"].T], axis=-1) for it in items]), np.float32)
+    om_t = np.ascontiguousarray(np.stack([it["omega"].T for it in items]), np.float32)
+    idx = np.arange(n, dtype=np.float32)
+    kv = np.ascontiguousarray(np.stack([(np.pi * (np.float32(2) * idx - np.float32(n)).astype(np.float64)
+                                         / np.float64(np.float32(it["tile_length"]))).astype(np.float32)
+                                        for it in items]))
+
+    def omega0(it):
+        per = it.get("anim_period", 200.0)
+        return 0.0 if per is None else float(np.float32(np.float64(np.float32(2.0)) * np.pi / np.float64(np.float32(per))))
+
+    om0 = np.array([omega0(it) for it in items], np.float32)
+    lam = np.array([it["lam"] for it in items], np.float32)
+    t = np.array([it["t"] for it in items], np.float32)
+    tex = np.float16 if half else np.float32
+    disp = np.zeros((k, n, n, 4), tex)
+    norm = np.zeros((k, n, n, 4), tex)
+    mm = np.zeros((k, 2), np.float32)
+    a = np.zeros(k, np.float32)
+    w = np.zeros((k, n // 2, 4, n), np.complex64) if want_w else None
+    p = lambda x: None if x is None else x.ctypes.data_as(C.c_void_p)
+    rc = lib().wso_emu_compute_shipped(logn, kind, 1 if half else 0, k, p(amp_t), p(om_t), p(kv), p(om0), p(lam), p(t),
+                                       p(disp), p(norm), p(mm), p(a), p(w))
+    if rc != 0:
+        raise ValueError(f"no emulated launch for logn={logn} kind={kind} (rc={rc})")
+    if w is not None and logn in PAIRED_W_LOGN:
+        w = np.concatenate([w[..., 0::2], w[..., 1::2]], axis=-1)
+    return a, disp.astype(np.float32), norm.astype(np.float32), mm[:, 0], mm[:, 1], w
 
 
 def compute_slab(n, tile_length, lam, h0_re, h0_im, omega, t, world, variant=0, anim_period=200.0):

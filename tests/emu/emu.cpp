@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "wso_kernels.cuh"
+#include "wso_tilings.h"
 
 using namespace wso;
 
@@ -463,4 +464,211 @@ extern "C" int wso_emu_compute(int logn, int variant, const float* amp_t, const 
     JCFG(10, 0, 4, 2, 4)
 #undef JCFG
     return -1;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// The tilings the library ships (wso_tilings.h), run as launch_tiled() / launch_tiled_jacobian() in wso_kernels.cu run
+// them: one launch of n_items tile-frames, item i with its own spectrum, wave numbers, lambda and time, written to slot i.
+// ---------------------------------------------------------------------------------------------------------------------
+
+// Same records, table and pair decision as upload_h0() in wso_api.cu; returns the tile constants.
+static TileDev make_tile(int N, const float* amp_t, const float* omega_t, const float* kv, float omega0, float lambda,
+                         std::vector<float4>& rec, std::vector<float4>& recs) {
+    const size_t n2 = (size_t)N * N;
+    int jmax = 0;
+    bool table_ok = omega0 > 0.0f;
+    for (size_t i = 0; i < n2 && table_ok; ++i) {
+        const float jf = std::nearbyint(omega_t[i] / omega0);
+        if (!(jf >= 0.0f && jf < (float)kMaxTable) || jf * omega0 != omega_t[i]) table_ok = false;
+        else if ((int)jf > jmax) jmax = (int)jf;
+    }
+    rec.assign(n2, make_float4(0.f, 0.f, 0.f, 0.f));
+    for (int n = 0; n < N; ++n)
+        for (int m = 0; m < N; ++m) {
+            const size_t i = (size_t)n * N + m;
+            const float d = kv[n] * kv[n] + kv[m] * kv[m];
+            const float inv = std::sqrt(d) > 0.00001f ? 1.0f / std::sqrt(d) : 0.0f;
+            float wf = omega_t[i];
+            if (table_ok) {
+                const int j = (int)std::nearbyint(omega_t[i] / omega0);
+                std::memcpy(&wf, &j, 4);
+            }
+            rec[h0_index(n, m, N, 0)] = make_float4(amp_t[2 * i], amp_t[2 * i + 1], inv, wf);
+        }
+    const int hN = N / 2;
+    recs.assign((size_t)hN * hN * 2, make_float4(0.f, 0.f, 0.f, 0.f));
+    bool pairs_ok = true;
+    for (int j = 1; j < hN; ++j)
+        for (int i = 1; i < hN; ++i) {
+            const float4 a0 = rec[h0_index(j, i, N, 0)], a3 = rec[h0_index(N - j, N - i, N, 0)];
+            const float4 a1 = rec[h0_index(N - j, i, N, 0)], a2 = rec[h0_index(j, N - i, N, 0)];
+            if (std::memcmp(&a0.w, &a3.w, 4) != 0 || std::memcmp(&a1.w, &a2.w, 4) != 0) pairs_ok = false;
+            recs[hs_index(j, i, 0, hN)] = make_float4(a0.x + a3.x, a0.y + a3.y, a0.z, a0.w);
+            recs[hs_index(j, i, 1, hN)] = make_float4(a1.x + a2.x, a1.y + a2.y, a1.z, a1.w);
+        }
+    TileDev td;
+    std::memset(&td, 0, sizeof(td));
+    td.h0 = rec.data();
+    td.hs = recs.data();
+    td.kv = kv;
+    td.lambda = lambda;
+    td.omega0 = omega0;
+    td.table_len = table_ok ? jmax + 1 : 0;
+    td.use_pairs = pairs_ok ? 1 : 0;
+    td.j0 = 0;
+    return td;
+}
+
+// PERSIST: bit 0 = K1, bit 2 = K2 in their persistent forms, taken - as in launch_tiled() - only where PersistOk allows
+// them and every item has the table and the pair records.  JAC: launch_tiled_jacobian() (general K1, one row item per K2
+// CTA).  amp_t / omega_t / kv: [n_items] consecutive arrays of the layout wso_emu_compute takes.
+template <int LOGN, class TL, bool JAC, int PERSIST, class TEX>
+static int run_launch(int n_items, const float* amp_t, const float* omega_t, const float* kv, const float* omega0,
+                      const float* lambda, const float* t, void* disp, void* norm, float* minmax, float* amp_out,
+                      float* w_out) {
+    constexpr int N = 1 << LOGN, H = N / 2;
+    const size_t n2 = (size_t)N * N;
+    if (n_items < 1 || n_items > LaunchArgs::kCap) return -3;
+    using P1 = Pass1<LOGN, TL::CP, TL::NF, false, false, JAC>;
+    using P1F = Pass1<LOGN, TL::CP, TL::NF, false, true>;
+    using P2 = Pass2<LOGN, JAC ? 1 : TL::RI, false, false, false, JAC, TEX>;
+    using PH = Pass2<LOGN, TL::RH, true>;
+    constexpr int RI2 = JAC ? 1 : TL::RI;
+    std::vector<float2> tw(N);
+    for (int k = 0; k < N; ++k) {
+        const double a = 2.0 * 3.14159265358979323846 * k / N;
+        tw[k] = make_float2((float)cos(a), (float)sin(a));
+    }
+    std::vector<std::vector<float4>> rec(n_items), recs(n_items);
+    std::vector<float2> W((size_t)n_items * H * 4 * N);
+    LaunchArgs args;
+    std::memset(&args, 0, sizeof(args));
+    bool fast = !JAC;
+    for (int i = 0; i < n_items; ++i) {
+        args.td[i] = make_tile(N, amp_t + 2 * n2 * i, omega_t + n2 * i, kv + (size_t)N * i, omega0[i], lambda[i], rec[i], recs[i]);
+        fast = fast && args.td[i].table_len > 0 && args.td[i].use_pairs != 0;
+        args.items[i].tile = (uint32_t)i;
+        args.items[i].slot = (uint32_t)i;
+        args.items[i].t = t[i];
+    }
+    args.tw = tw.data();
+    args.W = W.data();
+    args.disp = reinterpret_cast<float4*>(disp);
+    args.norm = reinterpret_cast<float4*>(norm);
+    args.minmax = minmax;
+    args.amp_out = amp_out;
+    constexpr bool p1 = (PERSIST & 1) && PersistOk<LOGN, TL>::k1, p2 = (PERSIST & 4) && PersistOk<LOGN, TL>::k2;
+    {   // K1
+        std::vector<float2> smem(P1::SMEM_BYTES / sizeof(float2));
+        std::vector<ThreadState> st(P1::T);
+        if (p1 && fast) {
+            if constexpr (p1) {
+                const int ncta = 5;
+                for (int cta = 0; cta < ncta; ++cta) {
+                    for (auto& v : smem) v = make_float2(NAN, NAN);
+                    for (auto& x : st) for (auto& v : x.v) v = make_float2(NAN, NAN);
+                    HostExec ex{P1::T, st.data()};
+                    P1F::run_persistent(ex, smem.data(), cta, ncta, n_items, args);
+                }
+            }
+        } else {
+            for (int bz = 0; bz < n_items; ++bz)
+                for (int by = 0; by < 4 / TL::NF; ++by)
+                    for (int bx = 0; bx < H / TL::CP; ++bx) {
+                        for (auto& v : smem) v = make_float2(NAN, NAN);
+                        HostExec ex{P1::T, st.data()};
+                        if (fast) P1F::run(ex, smem.data(), bx, by, bz, args);
+                        else P1::run(ex, smem.data(), bx, by, bz, args);
+                    }
+        }
+    }
+    if (w_out) std::memcpy(w_out, W.data(), W.size() * sizeof(float2));
+    {   // K2h: height extrema
+        std::vector<float2> smem(PH::SMEM_BYTES / sizeof(float2));
+        std::vector<ThreadState> st(PH::T);
+        for (int bz = 0; bz < n_items; ++bz)
+            for (int bx = 0; bx < PH::grid_x(); ++bx) {
+                for (auto& v : smem) v = make_float2(NAN, NAN);
+                HostExec ex{PH::T, st.data()};
+                PH::run(ex, smem.data(), bx, 0, bz, args);
+            }
+    }
+    {   // K2
+        std::vector<float2> smem(P2::SMEM_BYTES / sizeof(float2));
+        std::vector<ThreadState> st(P2::T);
+        if (p2 && fast) {
+            if constexpr (p2) {
+                const int ncta = 7;
+                for (int cta = 0; cta < ncta; ++cta) {
+                    for (auto& v : smem) v = make_float2(NAN, NAN);
+                    for (auto& x : st) for (auto& v : x.v) v = make_float2(NAN, NAN);
+                    HostExec ex{P2::T, st.data()};
+                    P2::run_persistent(ex, smem.data(), cta, ncta, n_items, args);
+                }
+            }
+        } else {
+            for (int bz = 0; bz < n_items; ++bz)
+                for (int by = 0; by < (JAC ? 1 : 2); ++by)
+                    for (int bx = 0; bx < H / RI2; ++bx) {
+                        for (auto& v : smem) v = make_float2(NAN, NAN);
+                        HostExec ex{P2::T, st.data()};
+                        P2::run(ex, smem.data(), bx, by, bz, args);
+                    }
+        }
+    }
+    return 0;
+}
+
+// kind: 0 = Cfg<L>::Lat, 1 = Cfg<L>::Bulk, 2 = Bulk with the persistent K1 and K2 where PersistOk allows them,
+// 3 = the Jacobian launch (Bulk tiling).  Sizes 16^2 ... 2048^2.
+enum { kEmuLat = 0, kEmuBulk = 1, kEmuPersist = 2, kEmuJacobian = 3, kEmuKinds = 4 };
+constexpr int kEmuMinLogN = 4, kEmuMaxLogN = 11;
+
+template <int LOGN, class TEX>
+static int shipped(int kind, int n_items, const float* amp_t, const float* omega_t, const float* kv, const float* omega0,
+                   const float* lambda, const float* t, void* disp, void* norm, float* minmax, float* amp_out, float* w_out) {
+    using B = typename Cfg<LOGN>::Bulk;
+    using L = typename Cfg<LOGN>::Lat;
+    switch (kind) {
+        case kEmuLat: return run_launch<LOGN, L, false, 0, TEX>(n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out);
+        case kEmuBulk: return run_launch<LOGN, B, false, 0, TEX>(n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out);
+        case kEmuPersist:
+            if (!(PersistOk<LOGN, B>::k1 || PersistOk<LOGN, B>::k2)) return -1;
+            return run_launch<LOGN, B, false, 5, TEX>(n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out);
+        case kEmuJacobian: return run_launch<LOGN, B, true, 0, TEX>(n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out);
+        default: return -1;
+    }
+}
+
+// half = 0: disp / norm receive [n_items][N*N] RGBA32F texels, half = 1: RGBA16F texels (4 x binary16).
+extern "C" int wso_emu_compute_shipped(int logn, int kind, int half, int n_items, const float* amp_t, const float* omega_t,
+                                       const float* kv, const float* omega0, const float* lambda, const float* t,
+                                       void* disp, void* norm, float* minmax, float* amp_out, float* w_out) {
+#define SHIP(L)                                                                                                              \
+    if (logn == L)                                                                                                       \
+        return half ? shipped<L, Half4>(kind, n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out) \
+                    : shipped<L, float4>(kind, n_items, amp_t, omega_t, kv, omega0, lambda, t, disp, norm, minmax, amp_out, w_out);
+    SHIP(4) SHIP(5) SHIP(6) SHIP(7) SHIP(8) SHIP(9) SHIP(10) SHIP(11)
+#undef SHIP
+    return -1;
+}
+
+// The tilings launch_all() can pick, from the same header as the library.  Row r = 7 ints: logn, kind (0 = Lat,
+// 1 = Bulk), CP, NF, RI, RH, persistent forms of Bulk (bit 0 = K1, bit 2 = K2).  Returns the row count (two per size,
+// logn 4 ... 13; wso_emu_compute_shipped runs logn 4 ... 11 of them).
+template <int LOGN>
+static int tiling_rows(int* out) {
+    using B = typename Cfg<LOGN>::Bulk;
+    using L = typename Cfg<LOGN>::Lat;
+    const int pm = (PersistOk<LOGN, B>::k1 ? 1 : 0) | (PersistOk<LOGN, B>::k2 ? 4 : 0);
+    const int rows[2][7] = {{LOGN, 0, L::CP, L::NF, L::RI, L::RH, 0}, {LOGN, 1, B::CP, B::NF, B::RI, B::RH, pm}};
+    std::memcpy(out, rows, sizeof(rows));
+    return 2;
+}
+extern "C" int wso_emu_tilings(int* out) {
+    int n = 0;
+#define ROWS(L) n += tiling_rows<L>(out + 7 * n);
+    ROWS(4) ROWS(5) ROWS(6) ROWS(7) ROWS(8) ROWS(9) ROWS(10) ROWS(11) ROWS(12) ROWS(13)
+#undef ROWS
+    return n;
 }
