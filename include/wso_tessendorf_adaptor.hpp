@@ -138,6 +138,14 @@ public:
         const uint32_t slot = 0;
         Check(wso_raycast_surface_host(m_Ctx, 1, &slot, &p, n, rays, out), "wso_raycast_surface_host");
     }
+    // Extension: the wave spectrum Prepare() builds (wsocean.h, "Wave spectra"): Pierson-Moskowitz, JONSWAP or TMA with
+    // finite depth and a wave-number band instead of the reference's Phillips spectrum; takes effect at the next Prepare().
+    void SetSpectrum(const wso_spectrum& s) { Check(wso_set_spectrum(m_Ctx, 0, &s), "wso_set_spectrum"); }
+    wso_spectrum GetSpectrum() const {
+        wso_spectrum s;
+        Check(wso_get_spectrum(m_Ctx, 0, &s), "wso_get_spectrum");
+        return s;
+    }
 
     // ---- extensions: device pointers for zero-copy consumers (e.g. Vulkan external memory, row f-2)
     void* GetDisplacementsDevice() const { return DevicePtr(WSO_MAP_DISPLACEMENT); }

@@ -285,6 +285,71 @@ WSO_API int wso_raycast_surface_host(wso_ctx* ctx, uint32_t n_slots, const uint3
                                      uint32_t n, const float* rays_host, wso_ray_hit* out_host);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Wave spectra (an extension): the sea state of a tile named by empirical numbers - wind speed, fetch, water depth, peak
+ * enhancement - instead of the reference's Phillips constant, with a wave-number band so that the cascades of a
+ * multi-tile context (tiles of different tile_length whose heights add up, as the surface queries and ray casts sum
+ * them) each carry their own part of ONE sea.  The spectrum is per tile and takes effect at the tile's next Prepare, like
+ * tile_length; all four Prepare entry points (wso_prepare, wso_prepare_gauss, wso_prepare_gauss_device,
+ * wso_prepare_counter) honour it, wso_import_h0* does not (the caller supplies the records).  Wind speed U and direction
+ * w^ come from wso_params as the setters store them; non-Phillips kinds ignore phillips_const and damping (the band
+ * replaces damping).  The sea stays point-symmetric: heightAmp_conj == conj(heightAmp) and omega depends on |k| only,
+ * so the per-frame kernels run unchanged.  Not on the slab path (wso_slab_*), which keeps the Phillips spectrum.
+ *   WSO_SPECTRUM_PHILLIPS (default): the reference's spectrum, built exactly as without this section; only the default
+ *       values of the other fields are accepted with it.
+ * Formulas (g = 9.81; "fl" = one fp32 rounding; every float64 operation is one IEEE operation in the order written, no
+ * FMA; exp, pow, tanh, lgamma are the C library's, so a device build may differ from the host build by 1 ulp in
+ * amplitude).  Per wave vector (kx, kz) of the grid (as wso_prepare):
+ *   fp32, as the Phillips build: dot = fl(kx*kx + kz*kz) (two products, one sum), k = fl(sqrt(dot)), inv = fl(1/k),
+ *       ux = fl(kx*inv), uz = fl(kz*inv).  k <= 1e-5: the record is zero (dispersion 0).
+ *   band: k_min <= k < k_max (fp32 comparison) carries energy; outside it P = 0.  Everything below is float64 on k, ux, uz.
+ *   dispersion: d = +inf: omega = sqrt(g*k), c_g = g/(2*omega).  Finite d: kd = k*d, th = tanh(kd),
+ *       omega = sqrt((g*k)*th), c_g = (g*(th + kd*(1 - th*th)))/(2*omega).
+ *   S(omega), r = omega_p/omega, r4 = (r*r)*(r*r): r4 >= 1400 gives S = 0 (underflow guard); else
+ *       S = (alpha*g*g * ((w2*w2)*w)) * exp(-1.25*r4), w = 1/omega, w2 = w*w                          (Pierson-Moskowitz shape)
+ *     PIERSON_MOSKOWITZ: alpha = 0.0081, omega_p = 0.855*g/U; U is the wind speed at 19.5 m above the sea.
+ *     JONSWAP: alpha = 0.076*pow(U*U/(F*g), 0.22), omega_p = 22*cbrt(g*g/(U*F)) (U at 10 m, F = fetch), and
+ *       S *= pow(gamma, exp(-(dw*dw)/(2*(so*so)))), dw = omega - omega_p, so = sigma*omega_p, sigma = 0.07 for
+ *       omega <= omega_p, else 0.09.
+ *     TMA: JONSWAP times Kitaigorodskii's Phi(wh), wh = omega*sqrt(d/g): Phi = 0.5*wh*wh for wh <= 1,
+ *       1 - 0.5*(2 - wh)^2 for wh < 2, else 1 (d = +inf: Phi = 1, TMA equals JONSWAP).
+ *   spreading D = (0.5*Q(s)) * (pow(0.5*(1 + c), s) + pow(0.5*(1 - c), s)), c = ux*w^x + uz*w^z clamped to [-1, 1]:
+ *       Hasselmann's Q(s)|cos(theta/2)|^2s made even in k; integrates to 1 over theta.
+ *       Q(s) = exp((2s - 1)*ln 2 + 2*lgamma(s + 1) - lgamma(2s + 1) - ln pi).
+ *       spread > 0: s = spread.  spread = 0: x = omega/omega_p, s = 6.97*pow(x, 4.06) for omega <= 1.05*omega_p,
+ *       else 9.77*pow(x, mu), mu = -2.33 - 1.45*(U*omega_p/g - 1.17).
+ *   energy P = (scale*dk*dk) * (((S*D)*c_g)/k), dk = 2*pi/L: the mean square height the wave vector contributes,
+ *       so E[mean h^2] = sum P and Hs = 4*sqrt(sum P) over the tile's band (see INTEGRATION.md §5, "Cascades").
+ *   amplitude s_amp = fl(min(sqrt(P), 2^64)) for P > 0, else 0 (also for the NaN of 0*inf at absurd inputs); re = fl(fl(inv_sqrt2*xi_re)*s_amp), im likewise (the Phillips build's
+ *       products, inv_sqrt2 = fl(1/fl(sqrt(2)))); heightAmp_conj = (re, -im).
+ *   dispersion stored: 0 where s_amp == 0, else fl(float(j)*omega0), omega0 = fl(2*pi/T) (frames loop with period T):
+ *       d = +inf: j = floor(fl(fl(sqrt(fl(9.81f*k))) / omega0)) in fp32 - the Phillips tile's j bit for bit;
+ *       finite d: j = floor(omega/omega0) in float64.  S is evaluated at the continuous omega.
+ * Device Prepare of a non-Phillips tile: one kernel; the per-frame sincos table is used when the largest in-band |k|
+ * quantises to j < 1024, otherwise the records hold omega and K1 evaluates sincos per wave vector (no size limit).
+ * WSO_ERR_INVALID_ARG (state unchanged): an unknown kind; fetch not finite > 0; depth not > 0 (+inf allowed); gamma not
+ * finite >= 1; spread not finite >= 0; k_min not finite >= 0; k_max NaN or <= k_min; scale not finite >= 0; PHILLIPS
+ * with any field other than its default.
+ * wso_spectrum_h0: the host build of the same records, no GPU needed (as wso_counter_h0): rows [m0, m0 + rows) of the
+ * N*N grid, xi = the full N*N complex array (re, im) of wso_prepare_gauss, or NULL = the counter generator (seed) of
+ * wso_prepare_counter.  m0 + rows must not exceed N. */
+enum { WSO_SPECTRUM_PHILLIPS = 0, WSO_SPECTRUM_PIERSON_MOSKOWITZ = 1, WSO_SPECTRUM_JONSWAP = 2, WSO_SPECTRUM_TMA = 3 };
+typedef struct wso_spectrum {
+    uint32_t kind;       /* WSO_SPECTRUM_*                                                                       */
+    float fetch;         /* F, metres (JONSWAP / TMA), finite > 0                                               */
+    float depth;         /* d, metres, > 0; +inf = deep water: dispersion and (TMA) attenuation                 */
+    float gamma;         /* JONSWAP / TMA peak enhancement, finite >= 1                                         */
+    float spread;        /* 0 = Hasselmann's frequency-dependent s(omega); > 0 = constant s                     */
+    float k_min, k_max;  /* band: only k_min <= |k| < k_max carries energy; 0 / +inf = unlimited               */
+    float scale;         /* multiplies S, finite >= 0; 1 = the empirical level                                  */
+} wso_spectrum;
+/* PHILLIPS; fetch 1e5, depth +inf, gamma 3.3, spread 0, band [0, +inf), scale 1 */
+WSO_API int wso_default_spectrum(wso_spectrum* s);
+WSO_API int wso_set_spectrum(wso_ctx* ctx, uint32_t tile, const wso_spectrum* s);
+WSO_API int wso_get_spectrum(const wso_ctx* ctx, uint32_t tile, wso_spectrum* s);
+WSO_API int wso_spectrum_h0(const wso_params* p, const wso_spectrum* s, const float* xi, uint64_t seed,
+                            uint32_t m0, uint32_t rows, wso_h0_record* out);
+
+/* ------------------------------------------------------------------------------------------------------------
  * External-memory interop (SURVEY row f-2): the maps land in memory a Vulkan device can bind, so the renderer's
  * vkCmdCopyBufferToImage reads them where K2 wrote them.  Replaces: the two 16*N*N-byte memcpy calls into the mapped
  * staging buffer and the PCIe upload behind them (WaterSurfaceMesh.cpp:701-755, vulkan/Texture2D.cpp:175-226).

@@ -5,6 +5,11 @@ kentril0/WaterSurfaceRendering's `WSTessendorf`), hand-written sm_100a CUDA behi
     ws = WSTessendorf(512, 1000.0); ws.Prepare(seed=1234); A = ws.ComputeWaves(1.5)
 """
 from . import _lib  # noqa: F401
-from .surface import H0_DTYPE, RAY_HIT_DTYPE, SURFACE_SAMPLE_DTYPE, PinnedBuffer, WSTessendorf  # noqa: F401
+from ._lib import (WSO_SPECTRUM_JONSWAP, WSO_SPECTRUM_PHILLIPS, WSO_SPECTRUM_PIERSON_MOSKOWITZ,  # noqa: F401
+                   WSO_SPECTRUM_TMA)
+from .surface import (H0_DTYPE, RAY_HIT_DTYPE, SURFACE_SAMPLE_DTYPE, PinnedBuffer, WSTessendorf,  # noqa: F401
+                      make_spectrum, spectrum_h0)
 
-__all__ = ["WSTessendorf", "PinnedBuffer", "H0_DTYPE", "SURFACE_SAMPLE_DTYPE", "RAY_HIT_DTYPE"]
+__all__ = ["WSTessendorf", "PinnedBuffer", "H0_DTYPE", "SURFACE_SAMPLE_DTYPE", "RAY_HIT_DTYPE", "make_spectrum",
+           "spectrum_h0", "WSO_SPECTRUM_PHILLIPS", "WSO_SPECTRUM_PIERSON_MOSKOWITZ", "WSO_SPECTRUM_JONSWAP",
+           "WSO_SPECTRUM_TMA"]

@@ -62,6 +62,27 @@ class WsoParams(C.Structure):
     ]
 
 
+# wave spectra (wso_set_spectrum): kind of a wso_spectrum
+WSO_SPECTRUM_PHILLIPS = 0
+WSO_SPECTRUM_PIERSON_MOSKOWITZ = 1
+WSO_SPECTRUM_JONSWAP = 2
+WSO_SPECTRUM_TMA = 3
+
+
+class WsoSpectrum(C.Structure):
+    """struct wso_spectrum (include/wsocean.h)."""
+    _fields_ = [
+        ("kind", C.c_uint32),
+        ("fetch", C.c_float),
+        ("depth", C.c_float),
+        ("gamma", C.c_float),
+        ("spread", C.c_float),
+        ("k_min", C.c_float),
+        ("k_max", C.c_float),
+        ("scale", C.c_float),
+    ]
+
+
 class WsoRayParams(C.Structure):
     """struct wso_ray_params (include/wsocean.h)."""
     _fields_ = [
@@ -114,6 +135,11 @@ SYMBOLS = {
     # ray casts (first hit of a segment with the displaced surface, 1..4 cascades)
     "wso_raycast_surface": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
     "wso_raycast_surface_host": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
+    # wave spectra (Pierson-Moskowitz / JONSWAP / TMA, finite depth, wave-number bands)
+    "wso_default_spectrum": (_int, [C.POINTER(WsoSpectrum)]),
+    "wso_set_spectrum": (_int, [_vp, _u32, C.POINTER(WsoSpectrum)]),
+    "wso_get_spectrum": (_int, [_vp, _u32, C.POINTER(WsoSpectrum)]),
+    "wso_spectrum_h0": (_int, [_pp, C.POINTER(WsoSpectrum), _vp, C.c_uint64, _u32, _u32, _vp]),
     # external-memory interop (Vulkan side of the maps)
     "wso_set_exportable": (_int, [_vp, _int]),
     "wso_export_fd": (_int, [_vp, _int, C.POINTER(_int), C.POINTER(C.c_size_t)]),

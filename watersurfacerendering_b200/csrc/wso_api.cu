@@ -16,6 +16,7 @@
 #include "wso_kernels.cuh"
 #include "wso_launch.h"
 #include "wso_query.cuh"
+#include "wso_spectrum.cuh"
 #include "wsocean.h"
 
 static_assert(sizeof(wso_surface_sample) == 2 * sizeof(float4), "one query record = two float4 stores");
@@ -37,6 +38,9 @@ struct Tile {
     wso_params prepared;        // parameters the resident h0 was built with
     bool is_prepared = false;
     std::vector<wso_h0_record> h0;  // host copy in the reference layout (export / checkpoint)
+    wso_spectrum spectrum = wso::default_spectrum();           // as set (pending until the next prepare)
+    wso_spectrum prepared_spectrum = wso::default_spectrum();  // what the resident records were built with (the
+                                                               // default after an import: the caller's records)
 };
 
 // What a map slot holds, for the surface queries: whether a compute has written it since its maps were last reset, the
@@ -554,9 +558,12 @@ int enqueue_chunk(wso_ctx* c, uint32_t n_items, const uint32_t* tiles, const flo
 
 // Prepare() on the device (SURVEY row f-3): one kernel builds both record arrays of the tile from a Gaussian array
 // already in device memory (d_xi) or from the counter-based generator (d_xi == NULL).
+int prepare_spectrum_on_device(wso_ctx* c, uint32_t tile, const float2* d_xi, uint64_t seed);
+
 int prepare_on_device(wso_ctx* c, uint32_t tile, const float2* d_xi, uint64_t seed) {
     const uint32_t n = c->n;
     Tile& tl = c->tiles[tile];
+    if (!wso::spectrum_is_phillips(tl.spectrum)) return prepare_spectrum_on_device(c, tile, d_xi, seed);
     const wso::DerivedParams d = wso::derive_params(tl.params);
     std::vector<float> kv;
     wso::host_wave_numbers(n, tl.params.tile_length, kv);
@@ -592,6 +599,42 @@ int prepare_on_device(wso_ctx* c, uint32_t tile, const float2* d_xi, uint64_t se
     c->h_tiles[tile].use_pairs = 1;
     tl.h0.clear();  // the records live on the device only; wso_export_h0 reads them back
     tl.prepared = tl.params;
+    tl.prepared_spectrum = tl.spectrum;
+    tl.is_prepared = true;
+    return WSO_OK;
+}
+
+// Device Prepare of a non-Phillips spectrum (include/wsocean.h, "Wave spectra").  The host picks K1's body for the tile:
+// the sincos table when the largest in-band |k| quantises to j < kMaxTable, otherwise omega in the records and the
+// general body.
+int prepare_spectrum_on_device(wso_ctx* c, uint32_t tile, const float2* d_xi, uint64_t seed) {
+    const uint32_t n = c->n;
+    Tile& tl = c->tiles[tile];
+    std::vector<float> kv;
+    wso::host_wave_numbers(n, tl.params.tile_length, kv);
+    wso::SpectrumPrepareArgs a;
+    a.c = wso::spectrum_consts(tl.params, tl.spectrum);
+    if (!(a.c.omega0 > 0.0f)) return fail(c, WSO_ERR_INVALID_ARG, "device Prepare: base frequency is not positive");
+    const double jmax = wso::spectrum_max_j(a.c, kv);
+    a.table = jmax < (double)wso::kMaxTable ? 1 : 0;
+    a.j_cap = a.table ? (int)jmax : 0;
+    a.h0 = c->d_h0 + (size_t)n * n * tile;
+    a.hs = c->d_hs + ((size_t)n * n / 2) * tile;
+    a.kv = c->d_kv + (size_t)n * tile;
+    a.xi = d_xi;
+    a.seed_mixed = wso::counter_seed_mix(seed);
+    a.n = (int)n;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    WSO_CUDA(c, cudaMemcpyAsync(c->d_kv + (size_t)n * tile, kv.data(), sizeof(float) * n, cudaMemcpyHostToDevice, c->stream));
+    WSO_CUDA(c, wso::launch_prepare_spectrum(a, c->stream));
+    WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+    c->launches += 1;
+    c->h_tiles[tile].omega0 = a.c.omega0;
+    c->h_tiles[tile].table_len = a.table ? a.j_cap + 1 : 0;
+    c->h_tiles[tile].use_pairs = 1;
+    tl.h0.clear();
+    tl.prepared = tl.params;
+    tl.prepared_spectrum = tl.spectrum;
     tl.is_prepared = true;
     return WSO_OK;
 }
@@ -740,6 +783,37 @@ int wso_get_params(const wso_ctx* c, uint32_t tile, wso_params* p) {
     return WSO_OK;
 }
 
+int wso_default_spectrum(wso_spectrum* s) {
+    if (!s) return WSO_ERR_INVALID_ARG;
+    *s = wso::default_spectrum();
+    return WSO_OK;
+}
+
+int wso_set_spectrum(wso_ctx* c, uint32_t tile, const wso_spectrum* s) {
+    if (!c || !s) return WSO_ERR_INVALID_ARG;
+    if (tile >= c->max_tiles) return fail(c, WSO_ERR_INVALID_ARG, "tile index out of range");
+    if (!wso::spectrum_valid(*s)) return fail(c, WSO_ERR_INVALID_ARG, "invalid spectrum; unchanged");
+    c->tiles[tile].spectrum = *s;
+    return WSO_OK;
+}
+
+int wso_get_spectrum(const wso_ctx* c, uint32_t tile, wso_spectrum* s) {
+    if (!c || !s || tile >= c->max_tiles) return WSO_ERR_INVALID_ARG;
+    *s = c->tiles[tile].spectrum;
+    return WSO_OK;
+}
+
+int wso_spectrum_h0(const wso_params* p, const wso_spectrum* s, const float* xi, uint64_t seed, uint32_t m0,
+                    uint32_t rows, wso_h0_record* out) {
+    if (!p || !s || !out || !valid_tile_size(p->tile_size, nullptr) || !valid_params(*p) || !wso::spectrum_valid(*s))
+        return WSO_ERR_INVALID_ARG;
+    if ((uint64_t)m0 + rows > p->tile_size) return WSO_ERR_INVALID_ARG;
+    wso_params q = *p;
+    wso::normalise_like_setters(q, nullptr);
+    wso::host_spectrum_rows(q, *s, xi, seed, m0, rows, out);
+    return WSO_OK;
+}
+
 int wso_set_lambda(wso_ctx* c, uint32_t tile, float lambda) {
     if (!c || tile >= c->max_tiles || !std::isfinite(lambda)) return WSO_ERR_INVALID_ARG;
     c->tiles[tile].params.lambda = lambda;
@@ -774,8 +848,15 @@ int wso_prepare_gauss(wso_ctx* c, uint32_t tile, const float* xi) {
     if (rc != WSO_OK) return rc;
     if (!xi) return fail(c, WSO_ERR_INVALID_ARG, "xi is NULL");
     Tile& tl = c->tiles[tile];
-    wso::host_base_wave_heights(tl.params, xi, tl.h0);
-    return upload_h0(c, tile, tl.h0.data());
+    if (wso::spectrum_is_phillips(tl.spectrum)) {
+        wso::host_base_wave_heights(tl.params, xi, tl.h0);
+    } else {
+        tl.h0.resize((size_t)c->n * c->n);
+        wso::host_spectrum_rows(tl.params, tl.spectrum, xi, 0, 0, c->n, tl.h0.data());
+    }
+    rc = upload_h0(c, tile, tl.h0.data());
+    if (rc == WSO_OK) tl.prepared_spectrum = tl.spectrum;
+    return rc;
 }
 
 int wso_prepare_gauss_device(wso_ctx* c, uint32_t tile, const float* xi) {
@@ -806,7 +887,9 @@ int wso_import_h0(wso_ctx* c, uint32_t tile, const wso_h0_record* h0) {
     int rc = begin_prepare(c, tile);
     if (rc != WSO_OK) return rc;
     if (!h0) return fail(c, WSO_ERR_INVALID_ARG, "h0 is NULL");
-    return upload_h0(c, tile, h0);
+    rc = upload_h0(c, tile, h0);
+    if (rc == WSO_OK) c->tiles[tile].prepared_spectrum = wso::default_spectrum();
+    return rc;
 }
 
 int wso_export_h0(const wso_ctx* c, uint32_t tile, wso_h0_record* h0) {
@@ -845,7 +928,9 @@ int wso_import_h0_compact(wso_ctx* c, uint32_t tile, const float* h0_3f) {
         full[i].amp_conj_im = -h0_3f[3 * i + 1];
         full[i].dispersion = h0_3f[3 * i + 2];
     }
-    return upload_h0(c, tile, full.data());
+    rc = upload_h0(c, tile, full.data());
+    if (rc == WSO_OK) c->tiles[tile].prepared_spectrum = wso::default_spectrum();
+    return rc;
 }
 
 int wso_export_h0_compact(const wso_ctx* c, uint32_t tile, float* h0_3f) {

@@ -6,6 +6,10 @@
 #include <cmath>
 #include <cstdint>
 #include <cstdlib>
+#include <cstring>
+#include <limits>
+
+#include "wso_spectrum.cuh"
 
 #ifndef M_PI
 #define M_PI 3.14159265358979323846
@@ -158,6 +162,129 @@ void counter_gauss(uint64_t seed, uint64_t idx, float* re, float* im) {
     const double a = 2.0 * M_PI * u2;
     *re = (float)(r * std::cos(a));
     *im = (float)(r * std::sin(a));
+}
+
+wso_spectrum default_spectrum() {
+    wso_spectrum s;
+    s.kind = WSO_SPECTRUM_PHILLIPS;
+    s.fetch = 1.0e5f;
+    s.depth = std::numeric_limits<float>::infinity();
+    s.gamma = 3.3f;
+    s.spread = 0.0f;
+    s.k_min = 0.0f;
+    s.k_max = std::numeric_limits<float>::infinity();
+    s.scale = 1.0f;
+    return s;
+}
+
+bool spectrum_is_phillips(const wso_spectrum& s) { return s.kind == WSO_SPECTRUM_PHILLIPS; }
+
+bool spectrum_valid(const wso_spectrum& s) {
+    if (s.kind > WSO_SPECTRUM_TMA) return false;
+    if (s.kind == WSO_SPECTRUM_PHILLIPS) {
+        // the Phillips kind is today's Prepare, which reads none of these fields: only the defaults are accepted
+        const wso_spectrum d = default_spectrum();
+        return std::memcmp(&s, &d, sizeof(s)) == 0;
+    }
+    const auto finite = [](float x) { return std::isfinite(x); };
+    return finite(s.fetch) && s.fetch > 0.0f && s.depth > 0.0f && !std::isnan(s.depth) && finite(s.gamma) &&
+           s.gamma >= 1.0f && finite(s.spread) && s.spread >= 0.0f && finite(s.k_min) && s.k_min >= 0.0f &&
+           !std::isnan(s.k_max) && s.k_max > s.k_min && finite(s.scale) && s.scale >= 0.0f;
+}
+
+SpectrumConsts spectrum_consts(const wso_params& p, const wso_spectrum& s) {
+    const double g = spec::kG;
+    const double U = (double)p.wind_speed;
+    const double F = (double)s.fetch;
+    SpectrumConsts c;
+    c.kind = (int)s.kind;
+    c.deep = std::isinf(s.depth) ? 1 : 0;
+    c.wind_x = p.wind_dir_x;
+    c.wind_y = p.wind_dir_y;
+    c.inv_sqrt2 = 1.0f / std::sqrt(2.0f);
+    c.omega0 = derive_params(p).base_freq;
+    c.k_min = s.k_min;
+    c.k_max = s.k_max;
+    c.depth = c.deep ? 0.0 : (double)s.depth;
+    c.sqrt_d_over_g = c.deep ? 0.0 : std::sqrt(c.depth / g);
+    double alpha;
+    if (s.kind == WSO_SPECTRUM_PIERSON_MOSKOWITZ) {
+        alpha = 0.0081;
+        c.omega_p = 0.855 * g / U;                        // U: wind speed at 19.5 m
+    } else {
+        alpha = 0.076 * std::pow(U * U / (F * g), 0.22);  // U: wind speed at 10 m, F: fetch
+        c.omega_p = 22.0 * std::cbrt(g * g / (U * F));
+    }
+    c.alpha_g2 = alpha * g * g;
+    c.gamma = (double)s.gamma;
+    c.spread = (double)s.spread;
+    c.q_const = s.spread > 0.0f ? spreading_norm(c.spread) : 0.0;
+    c.split = 1.05 * c.omega_p;
+    c.mu = -2.33 - 1.45 * (U * c.omega_p / g - 1.17);
+    const double dk = 2.0 * M_PI / (double)p.tile_length;
+    c.amp_scale = (double)s.scale * (dk * dk);
+    return c;
+}
+
+double spectrum_max_j(const SpectrumConsts& c, const std::vector<float>& kv) {
+    // |kx| in ascending order: kv[N/2 + t] for t = 0 .. N/2-1 (>= 0), then |kv[0]| (kv[N-i] == -kv[i] exactly).  For a
+    // fixed kz the fp32 |k| is non-decreasing along this order, so the largest |kx| with |k| < k_max is a binary search.
+    const size_t n = kv.size(), h = n / 2;
+    std::vector<float> ax(h + 1);
+    for (size_t t = 0; t < h; ++t) ax[t] = kv[h + t];
+    ax[h] = -kv[0];
+    const auto klen = [](float kx, float kz) { return std::sqrt(kx * kx + kz * kz); };
+    float kbest = 0.0f;
+    for (size_t m = 0; m < n; ++m) {
+        const float kz = kv[m];
+        size_t lo = 0, hi = h + 1;  // first index with |k| >= k_max
+        while (lo < hi) {
+            const size_t mid = (lo + hi) / 2;
+            if (klen(ax[mid], kz) < c.k_max) lo = mid + 1;
+            else hi = mid;
+        }
+        if (lo == 0) continue;
+        const float k = klen(ax[lo - 1], kz);
+        if (k >= c.k_min && k > 0.00001f && k > kbest) kbest = k;
+    }
+    if (!(kbest > 0.0f)) return 0.0;
+    if (c.deep) return (double)std::floor(std::sqrt(9.81f * kbest) / c.omega0);
+    double omega, cg;
+    spectrum_dispersion(c, (double)kbest, &omega, &cg);
+    return std::floor(omega / (double)c.omega0);
+}
+
+void host_spectrum_rows(const wso_params& p, const wso_spectrum& s, const float* xi, uint64_t seed, uint32_t m0,
+                        uint32_t rows, wso_h0_record* out) {
+    const uint32_t n = p.tile_size;
+    std::vector<float> kv;
+    host_wave_numbers(n, p.tile_length, kv);
+    const bool phillips = spectrum_is_phillips(s);
+    const H0Builder hb(p);
+    const SpectrumConsts c = phillips ? SpectrumConsts{} : spectrum_consts(p, s);
+    for (uint32_t m = m0; m < m0 + rows; ++m)
+        for (uint32_t col = 0; col < n; ++col) {
+            const size_t idx = (size_t)m * n + col;
+            float xr, xim;
+            if (xi) {
+                xr = xi[2 * idx];
+                xim = xi[2 * idx + 1];
+            } else {
+                counter_gauss(seed, idx, &xr, &xim);
+            }
+            wso_h0_record& r = out[(size_t)(m - m0) * n + col];
+            if (phillips) {
+                r = hb.at(kv[col], kv[m], xr, xim);
+                continue;
+            }
+            float re, im, inv, jf;
+            spectrum_record(c, kv[col], kv[m], xr, xim, &re, &im, &inv, &jf);
+            r.amp_re = re;
+            r.amp_im = im;
+            r.amp_conj_re = re;
+            r.amp_conj_im = -im;
+            r.dispersion = jf * c.omega0;
+        }
 }
 
 }  // namespace wso

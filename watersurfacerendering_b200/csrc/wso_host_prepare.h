@@ -33,4 +33,19 @@ struct H0Builder {
 // counter-based standard-normal pair for wave vector index idx (see wso_host_prepare.cpp)
 void counter_gauss(uint64_t seed, uint64_t idx, float* re, float* im);
 
+// Wave spectra (include/wsocean.h, "Wave spectra"; per-wave-vector arithmetic in wso_spectrum.cuh).
+struct SpectrumConsts;
+wso_spectrum default_spectrum();
+bool spectrum_valid(const wso_spectrum& s);
+bool spectrum_is_phillips(const wso_spectrum& s);
+// p: setter-normalised parameters; s: a valid non-Phillips spectrum
+SpectrumConsts spectrum_consts(const wso_params& p, const wso_spectrum& s);
+// largest multiple j of omega0 any in-band wave vector of the grid kv x kv can be quantised to (0: none in band);
+// j is monotone in |k|, so this is j of the largest in-band |k|
+double spectrum_max_j(const SpectrumConsts& c, const std::vector<float>& kv);
+// records of rows [m0, m0+rows) of the N*N grid: xi = full N*N complex array, or NULL = counter_gauss(seed, m*N+n);
+// the Phillips kind goes through H0Builder (bit for bit what wso_prepare_gauss / wso_counter_h0 build)
+void host_spectrum_rows(const wso_params& p, const wso_spectrum& s, const float* xi, uint64_t seed, uint32_t m0,
+                        uint32_t rows, wso_h0_record* out);
+
 }  // namespace wso

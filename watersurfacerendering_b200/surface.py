@@ -28,6 +28,41 @@ def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+SPECTRUM_KINDS = {"phillips": L.WSO_SPECTRUM_PHILLIPS, "pierson_moskowitz": L.WSO_SPECTRUM_PIERSON_MOSKOWITZ,
+                  "jonswap": L.WSO_SPECTRUM_JONSWAP, "tma": L.WSO_SPECTRUM_TMA}
+
+
+def make_spectrum(kind="phillips", *, fetch: float = 1e5, depth: float = np.inf, gamma: float = 3.3,
+                  spread: float = 0.0, k_band=(0.0, np.inf), scale: float = 1.0) -> "L.WsoSpectrum":
+    """A struct wso_spectrum; ``kind`` is a WSO_SPECTRUM_* value or one of SPECTRUM_KINDS' names.  The defaults are
+    wso_default_spectrum's.  Validation happens in the library (wso_set_spectrum / wso_spectrum_h0)."""
+    s = L.WsoSpectrum()
+    s.kind = SPECTRUM_KINDS[kind.lower()] if isinstance(kind, str) else int(kind)
+    s.fetch, s.depth, s.gamma, s.spread = float(fetch), float(depth), float(gamma), float(spread)
+    s.k_min, s.k_max = float(k_band[0]), float(k_band[1])
+    s.scale = float(scale)
+    return s
+
+
+def spectrum_dict(s: "L.WsoSpectrum") -> dict:
+    return {"kind": int(s.kind), "fetch": s.fetch, "depth": s.depth, "gamma": s.gamma, "spread": s.spread,
+            "k_band": (s.k_min, s.k_max), "scale": s.scale}
+
+
+def spectrum_h0(params: "L.WsoParams", spectrum: "L.WsoSpectrum", xi: Optional[np.ndarray] = None, seed: int = 0,
+                m0: int = 0, rows: Optional[int] = None) -> np.ndarray:
+    """Host build of the spectrum records (wso_spectrum_h0), rows [m0, m0+rows) in the reference layout: from the
+    N*N Gaussian array ``xi`` (as PrepareWithGauss), or from the counter generator of PrepareCounterOnDevice (``seed``)."""
+    n = int(params.tile_size)
+    rows = n - m0 if rows is None else int(rows)
+    if xi is not None:
+        xi = np.ascontiguousarray(xi, np.complex64).reshape(n, n)
+    out = np.zeros((rows, n), H0_DTYPE)
+    L.check(L.load().wso_spectrum_h0(C.byref(params), C.byref(spectrum), _ptr(xi), int(seed), int(m0), rows,
+                                     out.ctypes.data_as(C.c_void_p)))
+    return out
+
+
 class PinnedBuffer:
     """Page-locked host memory (wso_alloc_host) exposed as a NumPy array."""
 
@@ -157,6 +192,19 @@ class WSTessendorf:
         v = C.c_int()
         L.check(self._lib.wso_get_compute_jacobian(self._h, C.byref(v)), self._h)
         return bool(v.value)
+
+    # ------------------------------------------------------------------ wave spectra
+    def set_spectrum(self, kind="phillips", tile: int = 0, **kw):
+        """Spectrum of ``tile`` from its next Prepare on (wso_set_spectrum): ``kind`` = "phillips" (default, the
+        reference's), "pierson_moskowitz", "jonswap" or "tma"; keywords fetch, depth, gamma, spread, k_band = (k_min,
+        k_max), scale as in make_spectrum."""
+        s = make_spectrum(kind, **kw)
+        L.check(self._lib.wso_set_spectrum(self._h, tile, C.byref(s)), self._h)
+
+    def get_spectrum(self, tile: int = 0) -> dict:
+        s = L.WsoSpectrum()
+        L.check(self._lib.wso_get_spectrum(self._h, tile, C.byref(s)), self._h)
+        return spectrum_dict(s)
 
     # ------------------------------------------------------------------ prepare
     def Prepare(self, seed: Optional[int] = None, tile: int = 0):
