@@ -138,6 +138,16 @@ public:
         const uint32_t slot = 0;
         Check(wso_raycast_surface_host(m_Ctx, 1, &slot, &p, n, rays, out), "wso_raycast_surface_host");
     }
+    // Extension: hydrostatic force and torque on n rigid bodies (host arrays: bodies, n_vertices x (x, y, z, unused) body
+    // coordinates, n_triangles x 3 indices), floating in the surface of slot 0 (wsocean.h, "Hydrostatic forces").
+    // Blocking.
+    void Hydrostatics(const wso_body* bodies, uint32_t n, const float* vertices, uint32_t n_vertices,
+                      const uint32_t* triangles, uint32_t n_triangles, wso_hydro_result* out,
+                      const wso_hydro_params& p) {
+        const uint32_t slot = 0;
+        Check(wso_hydrostatics_host(m_Ctx, 1, &slot, &p, n, bodies, n_vertices, vertices, n_triangles, triangles, out),
+              "wso_hydrostatics_host");
+    }
     // Extension: the wave spectrum Prepare() builds (wsocean.h, "Wave spectra"): Pierson-Moskowitz, JONSWAP or TMA with
     // finite depth and a wave-number band instead of the reference's Phillips spectrum; takes effect at the next Prepare().
     void SetSpectrum(const wso_spectrum& s) { Check(wso_set_spectrum(m_Ctx, 0, &s), "wso_set_spectrum"); }

@@ -285,6 +285,88 @@ WSO_API int wso_raycast_surface_host(wso_ctx* ctx, uint32_t n_slots, const uint3
                                      uint32_t n, const float* rays_host, wso_ray_hit* out_host);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Hydrostatic forces (an extension): the buoyancy force and torque on rigid bodies, each a closed (or open) triangle
+ * hull with a pose, floating in the displaced surface of the same 1..4 slots as the surface queries.  One launch for
+ * every body of a physics step, on the context's stream, behind the compute that wrote the maps.
+ * Model: hydrostatic pressure p = density * gravity * depth on the wetted part of the hull, depth measured vertically
+ * from each point up to the displaced surface above it (the usual real-time approximation for ships and floating
+ * objects).  Not modelled: the attenuation of the wave pressure with depth (Froude-Krylov), drag, slamming, added mass,
+ * the orbital velocities of the waves.  A caller adds those on top; the wetted area is reported for drag.
+ * Inputs:
+ *   wso_body (80 bytes): R = rotation (row-major, body -> world; a proper rotation: a reflection turns the hull inside
+ *       out and negates force and torque), t = position, c = center (the reference point, body coordinates, usually the
+ *       centre of mass), and the body's vertex range [vertex_first, +vertex_count) and triangle range
+ *       [triangle_first, +triangle_count) in the shared arrays.  Several bodies may share ranges with different poses.
+ *   vertices: n_vertices x 4 floats (x, y, z, unused), body coordinates.
+ *   triangles: n_triangles x 3 uint32 indices, relative to the body's vertex_first.  Winding: counter-clockwise seen
+ *       from outside, (b - a) x (c - a) points out of the hull.
+ * Per vertex v (fp32, round-to-nearest, in this order; "fl" = one rounding, R v row by row as
+ *   fl(fl(fl(R_i0 v0) + fl(R_i1 v1)) + fl(R_i2 v2))):
+ *       c_w = fl(t + R c) (once per body), e = fl(v - c), arm = R e, world = fl(c_w + arm),
+ *       H = the height wso_query_surface returns at (world.x, world.z) with the same slots and iterations (bit for bit),
+ *       depth = fl(H - world.y).  The vertex is wet when depth > 0.
+ *   Arms come from v - c, so the torque is as accurate far from the world origin as near it.
+ * Per triangle (float64 from here, every operation rounded once, nothing fused): the triangle (arm, depth per vertex)
+ *   is clipped where the depth, linear along each edge, is zero: X on edge p -> q (p wet, q dry) is
+ *   p + u (q - p) with u = d_p / (d_p - d_q), depth 0.  Rotating the vertices cyclically so that the vertex on its own
+ *   side of the waterline is a (then b, c):
+ *       no wet vertex: nothing;  all wet: (v0, v1, v2);  a alone wet: (a, X_ab, X_ac);
+ *       a alone dry: the quad (X_ba, b, c, X_ca) split along the diagonal b - X_ca into (X_ba, b, X_ca), (b, c, X_ca).
+ *   Each wet sub-triangle with arms y_i, depths d_i adds, in this order:
+ *       S = 1/2 (y1 - y0) x (y2 - y0), sd = (d0 + d1) + d2,
+ *       F'   = -(sd / 3) S
+ *       tau' = -((g x S) / 12), g = ((d0 y0 + d1 y1) + d2 y2) + sd ((y0 + y1) + y2)
+ *       area = sqrt((Sx^2 + Sy^2) + Sz^2)
+ *   (exact integrals of a pressure linear over the triangle: integral f g dA = A/12 (sum f_i g_i + sum f_i sum g_i)).
+ * Per body: triangle i goes to lane i mod 256; each lane adds its triangles in increasing i into zeroed sums; lane sums
+ *   are then combined by a fixed pairwise tree: for stride = 128, 64, ..., 1, lane j += lane j + stride (j < stride).
+ *   k = density * gravity in float64; force = fl32(k * sum F'), torque = fl32(k * sum tau'), wetted_area = fl32(sum area).
+ *   The torque is about c_w, in world axes; force and torque are in world axes.
+ * Record (32 bytes, wso_hydro_result): status
+ *   WSO_HYDRO_DRY        no vertex of the range is wet: zeros;
+ *   WSO_HYDRO_PARTIAL    some vertices are wet;
+ *   WSO_HYDRO_SUBMERGED  every vertex is wet;
+ *   WSO_HYDRO_INVALID    NaN fields: vertex_count is 0 or > 4096, triangle_count > 65536, a range reaches past
+ *                        n_vertices / n_triangles, a triangle index >= vertex_count, R, t or c has a non-finite
+ *                        component, or a vertex, an arm or a depth is not finite.  Bodies are checked one by one on the
+ *                        device: bad data is never a call error, and the other bodies are unaffected.
+ * wso_hydrostatics: bodies_dev (n_bodies), vertices_dev (n_vertices x 4 floats), triangles_dev (n_triangles x 3),
+ *   out_dev (n_bodies records) are device pointers; bodies, vertices and out 16-byte aligned, triangles 4-byte aligned;
+ *   asynchronous on the context's stream, ONE kernel launch.
+ * wso_hydrostatics_host: host pointers; blocking; stages through library-owned device memory grown on demand.
+ * WSO_ERR_INVALID_ARG (state unchanged): everything wso_query_surface rejects (slots, n_slots, iterations > 16), a NULL
+ * p, density or gravity negative or not finite, reserved != 0, n_bodies >= 2^31, a NULL or misaligned pointer (a
+ * pointer may be NULL when its count is 0).  n_bodies == 0 is a no-op.  Not on the slab path. */
+typedef struct wso_body {
+    float rotation[9];          /* row-major R, body -> world */
+    float position[3];          /* t */
+    float center[3];            /* c, body coordinates: the torque is about its world position t + R c */
+    uint32_t vertex_first, vertex_count;       /* 1..4096 vertices */
+    uint32_t triangle_first, triangle_count;   /* 0..65536 triangles */
+    uint32_t unused;
+} wso_body;
+typedef struct wso_hydro_params {
+    float density;          /* kg / m^3, finite and >= 0 (sea water: 1025) */
+    float gravity;          /* m / s^2, finite and >= 0 */
+    uint32_t iterations;    /* inversion steps of every height, 0..16 (as wso_query_surface) */
+    uint32_t reserved;      /* 0 */
+} wso_hydro_params;
+enum { WSO_HYDRO_DRY = 0, WSO_HYDRO_PARTIAL = 1, WSO_HYDRO_SUBMERGED = 2, WSO_HYDRO_INVALID = 3 };
+typedef struct wso_hydro_result {
+    float force[3];         /* world axes, N */
+    float wetted_area;      /* m^2 */
+    float torque[3];        /* about t + R c, world axes, N m */
+    uint32_t status;        /* WSO_HYDRO_* */
+} wso_hydro_result;
+WSO_API int wso_hydrostatics(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, const wso_hydro_params* p,
+                             uint32_t n_bodies, const wso_body* bodies_dev, uint32_t n_vertices, const float* vertices_dev,
+                             uint32_t n_triangles, const uint32_t* triangles_dev, wso_hydro_result* out_dev);
+WSO_API int wso_hydrostatics_host(wso_ctx* ctx, uint32_t n_slots, const uint32_t* slots, const wso_hydro_params* p,
+                                  uint32_t n_bodies, const wso_body* bodies_host, uint32_t n_vertices,
+                                  const float* vertices_host, uint32_t n_triangles, const uint32_t* triangles_host,
+                                  wso_hydro_result* out_host);
+
+/* ------------------------------------------------------------------------------------------------------------
  * Wave spectra (an extension): the sea state of a tile named by empirical numbers - wind speed, fetch, water depth, peak
  * enhancement - instead of the reference's Phillips constant, with a wave-number band so that the cascades of a
  * multi-tile context (tiles of different tile_length whose heights add up, as the surface queries and ray casts sum

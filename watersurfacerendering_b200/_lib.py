@@ -41,6 +41,18 @@ WSO_RAY_INVALID = 4
 # struct wso_ray_hit (include/wsocean.h): one 48-byte record per ray, the hit's wso_surface_sample flattened into it
 RAY_HIT_DTYPE = [("distance", "<f4"), ("x", "<f4"), ("z", "<f4"), ("status", "<u4")] + SURFACE_SAMPLE_DTYPE
 
+# hydrostatics (wso_hydrostatics): status of a wso_hydro_result
+WSO_HYDRO_DRY = 0
+WSO_HYDRO_PARTIAL = 1
+WSO_HYDRO_SUBMERGED = 2
+WSO_HYDRO_INVALID = 3
+
+# struct wso_body (include/wsocean.h): pose, reference point and ranges of one rigid body, 80 bytes
+BODY_DTYPE = [("rotation", "<f4", (9,)), ("position", "<f4", (3,)), ("center", "<f4", (3,)), ("vertex_first", "<u4"),
+              ("vertex_count", "<u4"), ("triangle_first", "<u4"), ("triangle_count", "<u4"), ("unused", "<u4")]
+# struct wso_hydro_result (include/wsocean.h): one 32-byte record per body
+HYDRO_RESULT_DTYPE = [("force", "<f4", (3,)), ("wetted_area", "<f4"), ("torque", "<f4", (3,)), ("status", "<u4")]
+
 STATUS_NAMES = {
     0: "WSO_OK", -1: "WSO_ERR_INVALID_ARG", -2: "WSO_ERR_BAD_TILE_SIZE", -3: "WSO_ERR_NOT_PREPARED",
     -4: "WSO_ERR_CUDA", -5: "WSO_ERR_OUT_OF_MEMORY", -6: "WSO_ERR_H0_NOT_CONJUGATE",
@@ -93,6 +105,16 @@ class WsoRayParams(C.Structure):
     ]
 
 
+class WsoHydroParams(C.Structure):
+    """struct wso_hydro_params (include/wsocean.h)."""
+    _fields_ = [
+        ("density", C.c_float),
+        ("gravity", C.c_float),
+        ("iterations", C.c_uint32),
+        ("reserved", C.c_uint32),
+    ]
+
+
 # every symbol include/wsocean.h declares: name -> (restype, argtypes)
 _vp, _u32, _f32, _int = C.c_void_p, C.c_uint32, C.c_float, C.c_int
 _pp = C.POINTER(WsoParams)
@@ -135,6 +157,9 @@ SYMBOLS = {
     # ray casts (first hit of a segment with the displaced surface, 1..4 cascades)
     "wso_raycast_surface": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
     "wso_raycast_surface_host": (_int, [_vp, _u32, _vp, C.POINTER(WsoRayParams), _u32, _vp, _vp]),
+    # hydrostatics (buoyancy force and torque on triangle hulls, 1..4 cascades)
+    "wso_hydrostatics": (_int, [_vp, _u32, _vp, C.POINTER(WsoHydroParams), _u32, _vp, _u32, _vp, _u32, _vp, _vp]),
+    "wso_hydrostatics_host": (_int, [_vp, _u32, _vp, C.POINTER(WsoHydroParams), _u32, _vp, _u32, _vp, _u32, _vp, _vp]),
     # wave spectra (Pierson-Moskowitz / JONSWAP / TMA, finite depth, wave-number bands)
     "wso_default_spectrum": (_int, [C.POINTER(WsoSpectrum)]),
     "wso_set_spectrum": (_int, [_vp, _u32, C.POINTER(WsoSpectrum)]),

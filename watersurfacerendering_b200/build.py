@@ -18,10 +18,10 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB_PATH = os.path.join(PKG_DIR, "libwsocean.so")
 
 SOURCES = ["wso_kernels.cu", "wso_kernels2.cu", "wso_slab_kernels.cu", "wso_prepare_kernels.cu", "wso_spectrum.cu",
-           "wso_query_kernels.cu",
+           "wso_query_kernels.cu", "wso_hydro.cu",
            "wso_api.cu", "wso_slab.cu", "wso_host_prepare.cpp"]
 HEADERS = ["wso_device.cuh", "wso_kernels.cuh", "wso_kernels2.cuh", "wso_simt.cuh", "wso_launch.h", "wso_host_prepare.h",
-           "wso_query.cuh", "wso_tilings.h", "wso_spectrum.cuh",
+           "wso_query.cuh", "wso_hydro.cuh", "wso_tilings.h", "wso_spectrum.cuh",
            "wso_counter_gauss.cuh"]
 
 NVCC_FLAGS = [

@@ -2,6 +2,7 @@
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -13,6 +14,7 @@
 #include <cuda.h>  // types of the virtual-memory API only; entry points come from cudaGetDriverEntryPoint
 
 #include "wso_host_prepare.h"
+#include "wso_hydro.cuh"
 #include "wso_kernels.cuh"
 #include "wso_launch.h"
 #include "wso_query.cuh"
@@ -23,6 +25,13 @@ static_assert(sizeof(wso_surface_sample) == 2 * sizeof(float4), "one query recor
 static_assert(sizeof(wso_ray_hit) == 48, "one ray record = three float4 stores");
 static_assert(WSO_RAY_INVALID == wso::kRayInvalid && WSO_RAY_UNRESOLVED == wso::kRayUnresolved && WSO_RAY_HIT == wso::kRayHit,
               "ray status codes of the C ABI and the kernel body");
+static_assert(sizeof(wso_body) == 80 && sizeof(wso::HydroBody) == 80 && offsetof(wso_body, vertex_first) == 60 &&
+                  offsetof(wso::HydroBody, vertex_first) == 60 && offsetof(wso_body, unused) == 76,
+              "wso_body and the kernel's HydroBody share one layout");
+static_assert(sizeof(wso_hydro_result) == 2 * sizeof(float4), "one hydrostatics record = two float4 stores");
+static_assert(WSO_HYDRO_DRY == wso::kHydroDry && WSO_HYDRO_PARTIAL == wso::kHydroPartial &&
+                  WSO_HYDRO_SUBMERGED == wso::kHydroSubmerged && WSO_HYDRO_INVALID == wso::kHydroInvalid,
+              "hydrostatics status codes of the C ABI and the kernel body");
 
 using wso::BatchItem;
 using wso::LaunchArgs;
@@ -1318,6 +1327,25 @@ int check_raycast(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso
     return WSO_OK;
 }
 
+// wso_hydrostatics' checks: those of the queries plus the pressure parameters and the body count.
+int check_hydro(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_hydro_params* p, uint32_t n_bodies,
+                wso::HydroArgs* a) {
+    if (!c) return WSO_ERR_INVALID_ARG;
+    if (!p) return fail(c, WSO_ERR_INVALID_ARG, "hydro params are NULL");
+    *a = wso::HydroArgs{};
+    const int rc = check_query(c, n_slots, slots, p->iterations, &a->q);
+    if (rc != WSO_OK) return rc;
+    if (!(p->density >= 0.0f && p->density <= FLT_MAX)) return fail(c, WSO_ERR_INVALID_ARG, "density must be finite and >= 0");
+    if (!(p->gravity >= 0.0f && p->gravity <= FLT_MAX)) return fail(c, WSO_ERR_INVALID_ARG, "gravity must be finite and >= 0");
+    if (p->reserved != 0) return fail(c, WSO_ERR_INVALID_ARG, "reserved must be 0");
+    if (n_bodies > (uint32_t)INT32_MAX) return fail(c, WSO_ERR_INVALID_ARG, "n_bodies must be < 2^31");
+    a->k = (double)p->density * (double)p->gravity;   // exact: two 24-bit significands
+    a->n = n_bodies;
+    return WSO_OK;
+}
+
+bool aligned(const void* p, size_t a) { return reinterpret_cast<uintptr_t>(p) % a == 0; }
+
 // The device staging of the blocking query / ray-cast forms: at least in_bytes and out_bytes, grown on demand.
 int grow_staging(wso_ctx* c, size_t in_bytes, size_t out_bytes) {
     if (in_bytes <= c->stage_in_bytes && out_bytes <= c->stage_out_bytes) return WSO_OK;
@@ -1415,6 +1443,65 @@ int wso_raycast_surface_host(wso_ctx* c, uint32_t n_slots, const uint32_t* slots
     c->launches += 1;
     WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_stage_out, sizeof(wso_ray_hit) * (size_t)n, cudaMemcpyDeviceToHost,
                                 c->stream));
+    WSO_CUDA(c, cudaStreamSynchronize(c->stream));
+    return WSO_OK;
+}
+
+int wso_hydrostatics(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_hydro_params* p, uint32_t n_bodies,
+                     const wso_body* bodies_dev, uint32_t n_vertices, const float* vertices_dev, uint32_t n_triangles,
+                     const uint32_t* triangles_dev, wso_hydro_result* out_dev) {
+    wso::HydroArgs a;
+    int rc = check_hydro(c, n_slots, slots, p, n_bodies, &a);
+    if (rc != WSO_OK) return rc;
+    if (n_bodies == 0) return WSO_OK;
+    if (!bodies_dev || !out_dev || (n_vertices && !vertices_dev) || (n_triangles && !triangles_dev))
+        return fail(c, WSO_ERR_INVALID_ARG, "bodies, vertices, triangles or out is NULL");
+    if (!aligned(bodies_dev, 16) || !aligned(vertices_dev, 16) || !aligned(triangles_dev, 4) || !aligned(out_dev, 16))
+        return fail(c, WSO_ERR_INVALID_ARG, "bodies, vertices or out is not 16-byte aligned, or triangles not 4-byte");
+    a.bodies = reinterpret_cast<const wso::HydroBody*>(bodies_dev);
+    a.vertices = reinterpret_cast<const float4*>(vertices_dev);
+    a.triangles = triangles_dev;
+    a.out = reinterpret_cast<float4*>(out_dev);
+    a.n_vertices = n_vertices;
+    a.n_triangles = n_triangles;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    WSO_CUDA(c, wso::launch_hydrostatics(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    return WSO_OK;
+}
+
+int wso_hydrostatics_host(wso_ctx* c, uint32_t n_slots, const uint32_t* slots, const wso_hydro_params* p,
+                          uint32_t n_bodies, const wso_body* bodies_host, uint32_t n_vertices, const float* vertices_host,
+                          uint32_t n_triangles, const uint32_t* triangles_host, wso_hydro_result* out_host) {
+    wso::HydroArgs a;
+    int rc = check_hydro(c, n_slots, slots, p, n_bodies, &a);
+    if (rc != WSO_OK) return rc;
+    if (n_bodies == 0) return WSO_OK;
+    if (!bodies_host || !out_host || (n_vertices && !vertices_host) || (n_triangles && !triangles_host))
+        return fail(c, WSO_ERR_INVALID_ARG, "bodies, vertices, triangles or out is NULL");
+    // bodies, vertices and triangles packed into the input staging at 16-byte aligned offsets
+    const size_t body_bytes = sizeof(wso_body) * (size_t)n_bodies;
+    const size_t vert_bytes = sizeof(float) * 4 * (size_t)n_vertices;
+    const size_t tri_bytes = sizeof(uint32_t) * 3 * (size_t)n_triangles;
+    const size_t vert_off = (body_bytes + 15) & ~(size_t)15;
+    const size_t tri_off = (vert_off + vert_bytes + 15) & ~(size_t)15;
+    WSO_CUDA(c, cudaSetDevice(c->device));
+    rc = grow_staging(c, tri_off + tri_bytes, sizeof(wso_hydro_result) * (size_t)n_bodies);
+    if (rc != WSO_OK) return rc;
+    char* in = static_cast<char*>(c->d_stage_in);
+    WSO_CUDA(c, cudaMemcpyAsync(in, bodies_host, body_bytes, cudaMemcpyHostToDevice, c->stream));
+    if (vert_bytes) WSO_CUDA(c, cudaMemcpyAsync(in + vert_off, vertices_host, vert_bytes, cudaMemcpyHostToDevice, c->stream));
+    if (tri_bytes) WSO_CUDA(c, cudaMemcpyAsync(in + tri_off, triangles_host, tri_bytes, cudaMemcpyHostToDevice, c->stream));
+    a.bodies = reinterpret_cast<const wso::HydroBody*>(in);
+    a.vertices = reinterpret_cast<const float4*>(in + vert_off);
+    a.triangles = reinterpret_cast<const uint32_t*>(in + tri_off);
+    a.out = static_cast<float4*>(c->d_stage_out);
+    a.n_vertices = n_vertices;
+    a.n_triangles = n_triangles;
+    WSO_CUDA(c, wso::launch_hydrostatics(a, (int)n_slots, c->map_format == WSO_MAP_RGBA16F, c->stream));
+    c->launches += 1;
+    WSO_CUDA(c, cudaMemcpyAsync(out_host, c->d_stage_out, sizeof(wso_hydro_result) * (size_t)n_bodies,
+                                cudaMemcpyDeviceToHost, c->stream));
     WSO_CUDA(c, cudaStreamSynchronize(c->stream));
     return WSO_OK;
 }

@@ -95,5 +95,9 @@ cudaError_t launch_query_surface(const QueryArgs& args, int n_slots, bool half, 
 // Ray casts (same files): one launch, one thread per ray over args.q.c[0..n_slots).  args.n > 0.
 struct RayArgs;
 cudaError_t launch_raycast_surface(const RayArgs& args, int n_slots, bool half, cudaStream_t stream);
+// Hydrostatics (wso_hydro.cu, body in wso_hydro.cuh): one launch, one 256-thread CTA per body over args.q.c[0..n_slots).
+// 1 <= args.n < 2^31.
+struct HydroArgs;
+cudaError_t launch_hydrostatics(const HydroArgs& args, int n_slots, bool half, cudaStream_t stream);
 
 }  // namespace wso

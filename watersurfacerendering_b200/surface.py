@@ -22,6 +22,10 @@ H0_DTYPE = np.dtype(
 SURFACE_SAMPLE_DTYPE = np.dtype(L.SURFACE_SAMPLE_DTYPE)
 # wso_ray_hit: distance, hit x / z, status (WSO_RAY_*), then the wso_surface_sample at (x, z)
 RAY_HIT_DTYPE = np.dtype(L.RAY_HIT_DTYPE)
+# wso_body: rotation (row-major, body -> world), position, center (reference point), vertex / triangle ranges
+BODY_DTYPE = np.dtype(L.BODY_DTYPE)
+# wso_hydro_result: force (world axes), wetted area, torque (about position + rotation @ center), status (WSO_HYDRO_*)
+HYDRO_RESULT_DTYPE = np.dtype(L.HYDRO_RESULT_DTYPE)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -419,6 +423,44 @@ class WSTessendorf:
         p = self._ray_params(step, max_steps, refine, iterations)
         L.check(self._lib.wso_raycast_surface(self._h, ns, _ptr(sl), C.byref(p), int(n), C.c_void_p(rays_ptr or 0),
                                               C.c_void_p(out_ptr or 0)), self._h)
+
+    # ---- hydrostatics (extension: buoyancy force and torque on triangle hulls, integrated on the device)
+    @staticmethod
+    def _hydro_params(iterations, density, gravity):
+        return L.WsoHydroParams(float(density), float(gravity), int(iterations), 0)
+
+    def hydrostatics(self, bodies, vertices, triangles, slots=(0,), iterations: int = 4, density: float = 1025.0,
+                     gravity: float = 9.81) -> np.ndarray:
+        """Hydrostatic force and torque on each body of `bodies` (BODY_DTYPE array, or one record), a triangle hull in
+        `vertices` ((n, 3) or (n, 4) body coordinates) and `triangles` ((m, 3) indices relative to each body's
+        vertex_first, counter-clockwise seen from outside), floating in the surface summed over the cascades `slots`
+        with `iterations` inversion steps per height.  Blocking (wso_hydrostatics_host).  -> structured array of records
+        (HYDRO_RESULT_DTYPE: force, wetted_area, torque about the body's world reference point, status = WSO_HYDRO_*)."""
+        b = np.ascontiguousarray(np.atleast_1d(np.asarray(bodies, BODY_DTYPE)))
+        v = np.atleast_2d(np.asarray(vertices, np.float32))
+        if v.ndim != 2 or v.shape[1] not in (3, 4):
+            raise ValueError("vertices must be an (n, 3) or (n, 4) array")
+        v4 = np.zeros((v.shape[0], 4), np.float32)
+        v4[:, :v.shape[1]] = v
+        t = np.ascontiguousarray(triangles, np.uint32).reshape(-1, 3)
+        out = np.zeros(b.shape[0], HYDRO_RESULT_DTYPE)
+        sl, ns = self._slots(slots)
+        p = self._hydro_params(iterations, density, gravity)
+        L.check(self._lib.wso_hydrostatics_host(self._h, ns, _ptr(sl), C.byref(p), b.shape[0], _ptr(b), v4.shape[0],
+                                                _ptr(v4), t.shape[0], _ptr(t), _ptr(out)), self._h)
+        return out
+
+    def hydrostatics_device(self, bodies_ptr: int, n_bodies: int, vertices_ptr: int, n_vertices: int,
+                            triangles_ptr: int, n_triangles: int, out_ptr: int, slots=(0,), iterations: int = 4,
+                            density: float = 1025.0, gravity: float = 9.81):
+        """The same on device memory (e.g. tensor.data_ptr()): n_bodies 80-byte wso_body records, n_vertices x 4 floats,
+        n_triangles x 3 uint32, out_ptr = n_bodies 32-byte records; bodies, vertices and out 16-byte aligned.
+        Asynchronous on the context's stream (wso_hydrostatics)."""
+        sl, ns = self._slots(slots)
+        p = self._hydro_params(iterations, density, gravity)
+        L.check(self._lib.wso_hydrostatics(self._h, ns, _ptr(sl), C.byref(p), int(n_bodies), C.c_void_p(bodies_ptr or 0),
+                                           int(n_vertices), C.c_void_p(vertices_ptr or 0), int(n_triangles),
+                                           C.c_void_p(triangles_ptr or 0), C.c_void_p(out_ptr or 0)), self._h)
 
     # ---- external-memory interop (SURVEY row f-2; replaces the staging memcpy of WaterSurfaceMesh.cpp:701-755)
     def set_exportable(self, on: bool = True):
